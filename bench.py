@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ssq_stft input Msamples/s on B200 (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 A step = one pass of the fused ssq_stft kernel over one batch of synthetic
 multichannel input.  N=1 workload = BASELINE.json configs[1]: 384 channels x
@@ -16,6 +16,9 @@ max-over-ranks device time.
 `--impl reference`: the reference's own algorithm on the host cores (the C
            restatement oracle/ssq_stft_ref.c, as-written variant; the Rust
            crate cannot be built in this image), rank 0 only, bounded sample.
+`--dump-outputs DIR`: after the timed steps, rank 0 writes a fixed, seeded
+           sample of the Tx its last step computed to DIR/Tx.npy (see
+           dump_outputs), so that two builds can be compared on the same input.
 """
 from __future__ import annotations
 
@@ -193,6 +196,26 @@ def make_neural_cpu(channels, n, fs, seed):
                   + 10 * np.sin(2 * np.pi * (40 + 20 * np.sin(2 * np.pi * 0.2 * t)) * t)
                   + 5 * np.sin(2 * np.pi * 60 * t) + 10 * rng.standard_normal(n) + sp)
     return out
+
+
+DUMP_COLUMNS = 16384  # x 257 bins x 8 bytes = 34 MB: a dump stays under 64 MB
+DUMP_SEED = 0x5351
+
+
+def dump_outputs(path, Tx):
+    """Writes a fixed sample of Tx [channels, n_freqs, n_frames] (complex64, on the device) to path/Tx.npy:
+    DUMP_COLUMNS (channel, frame) columns drawn without replacement by a generator seeded with DUMP_SEED, in
+    ascending (channel, frame) order, as float32 [columns, n_freqs, 2] (real, imaginary).  The columns depend only on
+    the shape of Tx, so two runs with the same arguments dump the same columns."""
+    import torch
+    ch, _, nfr = Tx.shape
+    k = min(DUMP_COLUMNS, ch * nfr)
+    flat = np.sort(np.random.default_rng(DUMP_SEED).choice(ch * nfr, size=k, replace=False))
+    c = torch.from_numpy(flat // nfr).to(Tx.device)
+    f = torch.from_numpy(flat % nfr).to(Tx.device)
+    cols = torch.view_as_real(Tx[c, :, f]).cpu().numpy()
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "Tx.npy"), cols.astype(np.float32, copy=False))
 
 
 def cpu_reference_run(n_samples, steps, warmup, mode=0, channels=1):
@@ -562,7 +585,7 @@ def run_reference(args, rank, world):
     if rank != 0:
         return
     n_s = args.ref_samples
-    steps = max(1, min(args.steps, 20))
+    steps = args.steps
     warm = max(1, min(args.warmup, 3))
     msps, threads, sec = cpu_reference_run(n_s, steps, warm, mode=0)
     line = {
@@ -642,6 +665,8 @@ def run_ours(args, rank, world, local_rank):
     chk = float(torch.view_as_real(Tx[0, :, :64]).abs().sum().item())
     if not np.isfinite(chk) or chk == 0.0:
         raise SystemExit("bench.py: kernel produced no output")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, Tx)
 
     # ---- roofline of the dominant kernel (live CUDA-event durations) -----------
     peak, peak_src = measured_peak_gbs()
@@ -924,14 +949,21 @@ def main():
                     help="ssq_stft (default, BASELINE configs[1]) is the contract line; the others time the "
                          "remaining rows of SURVEY 8 (configs[3] istft 4096 ch x 300 k, configs[2] ssq_cwt on a "
                          "channel cut of 2^20 samples, stft on configs[1]) with the same JSON layout")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="default workload only: write a seeded sample of the last timed step's Tx to DIR/Tx.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    other = args.workload != "ssq_stft" or (args.n_fft, args.hop) != (N_FFT, HOP)
+    if args.dump_outputs and (args.impl == "reference" or other):
+        ap.error("--dump-outputs is supported for the default workload (ssq_stft, n_fft 512, hop 32) only")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
         run_reference(args, rank, world)
-    elif args.workload != "ssq_stft" or (args.n_fft, args.hop) != (N_FFT, HOP):
+    elif other:
         run_other(args, rank, world, local_rank)
     else:
         run_ours(args, rank, world, local_rank)
