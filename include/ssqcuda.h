@@ -86,10 +86,10 @@ const char* ssq_last_error(const ssq_ctx* ctx);
 /* borrow a caller-owned cudaStream_t (NULL restores the context's own stream) */
 ssq_status ssq_ctx_set_stream(ssq_ctx* ctx, void* cuda_stream);
 ssq_status ssq_ctx_synchronize(ssq_ctx* ctx);
-/* kernel-selection switches for measurements and cross-checks (DESIGN.md 6c); none changes results beyond
- * fp32 rounding.  Every option is seeded once, at ssq_ctx_create, from the environment variable SSQ_<NAME>.
- * names: no_h32r, h32r_nw (4|8), no_r1024, no_r256, istft_nw (4|8), no_fft128, fft128_tc (32|64),
- * no_cwt_prune, no_cwt_fused, cwt_ws_mb.
+/* context options (DESIGN.md 6c); an unknown name returns SSQ_EINVAL.  Nothing reads them from the environment.
+ * Reference paths for cross-checks, none changes results beyond fp32 rounding: no_h32r, no_r1024, no_r256 (n_fft
+ * 512 / 1024 / 256 through the generic shared-memory kernels), no_cwt_fused (ssq_cwt through the ordered,
+ * bit-deterministic stand-alone reassignment).
  * One option does change results: upstream_framing = 1 frames the STFT family as upstream ssqueezepy does (left pad
  * n_fft / 2 instead of the crate's (n_fft - 1) / 2, stft_utils.rs:22) -- the upstream-compatible mode, SURVEY 8f rank 3. */
 ssq_status ssq_ctx_set_option(ssq_ctx* ctx, const char* name, int64_t value);

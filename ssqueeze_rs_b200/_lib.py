@@ -179,7 +179,9 @@ class Context:
         raise_status(load().ssq_ctx_set_stream(self._h, c_vp(cuda_stream_ptr or 0)), self._h)
 
     def set_option(self, name: str, value: int):
-        """Kernel-selection switch (measurements / cross-checks; include/ssqcuda.h ssq_ctx_set_option)."""
+        """Context option (include/ssqcuda.h ssq_ctx_set_option): ``no_h32r``, ``no_r1024``, ``no_r256`` and
+        ``no_cwt_fused`` select the reference paths of the cross-checks, ``upstream_framing`` the upstream framing.
+        An unknown name raises ValueError."""
         raise_status(load().ssq_ctx_set_option(self._h, name.encode(), int(value)), self._h)
 
     def synchronize(self):

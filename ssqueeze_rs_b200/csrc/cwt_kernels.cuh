@@ -409,7 +409,7 @@ __device__ __forceinline__ float2 tw_fwd(const FftPass& P, int64_t e) {  // W_L^
 // transform, bin and the update of Tx happen straight from the registers; Wx / dWx are never written.  The update is
 // a vector reduction (red.global.add.v2.f32): several scales may hit one Tx element from different CTAs, so the
 // order of additions inside an element is not fixed (rounding-level; the bins are).
-template <int TC, bool FUSED = false>  // TC adjacent columns per CTA (32 or 64): TC * 8 B contiguous per global access, 8 * TC threads
+template <int TC, bool FUSED = false>  // TC adjacent columns per CTA (16 or 32): TC * 8 B contiguous per global access, 8 * TC threads
 __global__ void __launch_bounds__(8 * TC) fft128_pass_kernel(const FftPass P) {
   extern __shared__ float2 buf[];  // [TC * 129]
   __shared__ float2 w128[128];  // W_128^m

@@ -11,7 +11,7 @@
 #pragma once
 #include "stft_kernels.cuh"
 
-template <bool PK = SSQ_PK_DEFAULT>
+template <bool PK = true>
 __device__ __forceinline__ void fft8_fwd(float2 (&v)[8]) {
   const float S = 0.70710678118654752440f;
   float2 a0 = caddf<PK>(v[0], v[4]), a4 = csubf<PK>(v[0], v[4]);
@@ -39,7 +39,7 @@ __device__ __forceinline__ void fft8_fwd(float2 (&v)[8]) {
 }
 
 // Same butterfly with the conjugate kernel: v[m] <- sum_t v[t] W_8^{-t m}.
-template <bool PK = SSQ_PK_DEFAULT>
+template <bool PK = true>
 __device__ __forceinline__ void fft8_inv(float2 (&v)[8]) {
   const float S = 0.70710678118654752440f;
   float2 a0 = caddf<PK>(v[0], v[4]), a4 = csubf<PK>(v[0], v[4]);
@@ -92,7 +92,7 @@ struct H32Lane {
 // ROT: the last butterfly of vb uses the conjugate kernel (see stft_h32r.cuh).
 // TW2POW: stage-2 twiddles by powers of one table entry (saves 12 shared-memory wavefronts, costs 24
 // multiplies: a gain where the data pipe binds -- stft/ssq_stft -- and a loss for istft).
-template <bool ROT = false, bool TW2POW = ROT, bool PK = SSQ_PK_DEFAULT>
+template <bool ROT = false, bool TW2POW = ROT, bool PK = true>
 __device__ __forceinline__ void h32_fft512(const H32Lane& L, float2* xch, float2 (&va)[8], float2 (&vb)[8]) {
   const int lane = L.lane, j2 = L.j2;
   fft8_fwd<PK>(va);

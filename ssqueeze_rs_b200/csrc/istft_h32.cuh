@@ -1,20 +1,15 @@
-// istft_h32.cuh -- inverse STFT for n_fft = 512 (BASELINE.json configs[3]: hop = 32; the tile kernel
-// that is launched takes any hop).
+// istft_h32.cuh -- inverse STFT for n_fft = 512, any hop (BASELINE.json configs[3]: hop = 32).
 //
 // old/ssqueezepy/_stft.py:184-256 in the Rust framing (unmodulated, unpad at
-// (n_fft-1)/2).  A warp owns a RUN of consecutive frames of one channel:
-//   * the columns Sx[:, f] of 4 frames are fetched with cp.async (32 B row
-//     segments, 8 rows per warp instruction) into a per-warp tile while the
-//     previous frames are being transformed;
+// (n_fft-1)/2):
 //   * two frames share one complex 512-point FFT: Z = ZA + i ZB with the Hermitian
 //     extension built on the fly, x_A = Re, x_B = Im of the inverse transform (the
 //     imaginary parts of the DC and Nyquist bins are dropped as irfft does);
-//   * overlap-add happens in a register window: with hop == warp size, sample
-//     n = lane + 32 j of frame f lands on padded position 32 (f + j) + lane, i.e. in
-//     the SAME lane for every frame, so a lane keeps 16 running sums, adds 16
-//     windowed samples per frame, emits the finished 128 B block and shifts;
-//   * blocks at the two ends of a run are shared with the neighbouring runs: every
-//     block is emitted with one red.global.add.f32 per lane into a zeroed buffer
+//   * with hop == warp size, sample n = lane + 32 j of frame f lands on padded position
+//     32 (f + j) + lane, i.e. in the SAME lane for every frame, so a warp adds its frames
+//     in a 16-register window;
+//   * samples at the two ends of a tile are shared with the neighbouring tiles: every
+//     sample is emitted with one red.global.add.f32 into a zeroed buffer
 //     (at most two addends per element: exact and order-independent);
 //   * istft_finalize_kernel divides by the window norm and unpads.
 #pragma once
@@ -40,24 +35,26 @@ struct Istft32Params {
   float* xacc;       // [channels, L] zero-initialised
   int run;           // frames per run (multiple of 4)
   int64_t runs_per_channel, total_runs;
-  int hop;           // tile kernel: any hop >= 1 (the per-warp-run kernel needs hop == 32)
+  int hop;           // any hop >= 1
+  int n_fft;         // host only: the launchers' guard
 };
 
-// Tile variant (the one launched): the per-warp quad fetch above leaves every 128 B line
-// of Sx "open" for four quads of one warp; with 2368 warps that is ~78 MB of partially
-// consumed lines, L2 thrashes and DRAM reads 2.2x the input (ncu r1f).  Here a CTA owns
-// 32 consecutive frames: the [257 x 32] tile is loaded with 256 B row segments, warp w
-// transforms frames 4w..4w+3 (two packed pairs) and parks the windowed samples in the
-// frame's own tile row; the overlap-add is a gather (each padded sample sums the <= 16
-// rows that cover it: no shared-memory atomics), one red.global.add per sample and tile.
+// A CTA owns 32 consecutive frames (a warp fetching its own quads of frames left every
+// 128 B line of Sx "open" for four quads of one warp; with 2368 warps that is ~78 MB of
+// partially consumed lines, L2 thrashed and DRAM read 2.2x the input: ncu r1f): the
+// [257 x 32] tile is loaded with 256 B row segments, warp w transforms frames 4w..4w+3
+// (two packed pairs) and parks the windowed samples in the frame's own tile row; the
+// overlap-add is a gather (each padded sample sums the <= 16 rows that cover it: no
+// shared-memory atomics), one red.global.add per sample and tile.
 // ------------------------------------------------------------------------------------
 #define I32T_AS 289  // tile row stride (float2): odd -> conflict-free transposed tile load; 578 floats >= 512
+// warps per CTA, tile = 4 NW = 32 frames, 2 CTAs per SM (4 warps x 16 frames, 4 CTAs per SM: 10.2 vs 9.5 ms)
+#define I32T_NW 8
 
-// NW warps per CTA, tile = 4 NW frames: 8 warps x 32 frames (2 CTAs per SM) or 4 warps x 16 frames (4 CTAs per SM: the
-// same 16 warps, but four independent CTAs interleave their load and transform phases and the barrier domain halves)
-template <bool HOP32, int NW>  // hop == 32: shifts instead of integer divisions in the gather
-__global__ void __launch_bounds__(NW * 32, 16 / NW) istft512_tile_kernel(const Istft32Params P) {
-  constexpr int N = 512, AS = I32T_AS, F = 4 * NW;
+template <bool HOP32>  // hop == 32: shifts instead of integer divisions in the gather
+__global__ void __launch_bounds__(I32T_NW * 32, 16 / I32T_NW) istft512_tile_kernel(const Istft32Params P) {
+  constexpr int N = 512, AS = I32T_AS, NW = I32T_NW, F = 4 * NW;
+  static_assert(F == 32, "the tile load maps lane -> frame and warp -> row: 8 warps x 32 frames");
   extern __shared__ float2 smem[];
   float2* tw2tab = smem;      // [8][9]
   float2* S = smem + 72;      // [32][AS]
@@ -92,10 +89,9 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) istft512_tile_kernel(const I
     const int ch = (int)(tile / P.runs_per_channel);
     const int64_t f0 = (tile % P.runs_per_channel) * F;
     const int nf = (int)min((int64_t)F, P.n_use - f0);
-    // ---- tile load: 8 rows per step; lane -> frame (F = 32: one row per warp, 256 B; F = 16: two rows per warp) ----
+    // ---- tile load: 8 rows per step; lane -> frame, one row per warp (256 B) ----
     {
-      const int fr = lane & (F - 1), rsub = (NW == 8) ? 0 : (lane >> 4);
-      const int r0 = (NW == 8) ? warp : 2 * warp + rsub;
+      const int fr = lane, r0 = warp;
       const float2* g = P.Sx + ((size_t)ch * 257 + r0) * P.n_frames + f0 + fr;
       const size_t gstep = (size_t)8 * P.n_frames;
       float2* s = S + fr * AS + r0;
@@ -226,4 +222,23 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) istft512_tile_kernel(const I
     }
     __syncthreads();
   }
+}
+
+static ssq_status istft512_launch(ssq_ctx* ctx, Istft32Params& Q, bool* done) {
+  *done = false;
+  // the tile span must stay inside the range of ssq_fast_div
+  if (Q.n_fft != 512 || ctx->opt.no_h32r || (int64_t)31 * Q.hop + 512 >= ((int64_t)1 << 22)) return SSQ_OK;
+  constexpr int NW = I32T_NW, F = 4 * NW;
+  Q.run = F;
+  Q.runs_per_channel = (Q.n_use + F - 1) / F;
+  Q.total_runs = Q.runs_per_channel * Q.channels;
+  *done = true;
+  const size_t smem = ((size_t)72 + (size_t)F * I32T_AS + (size_t)NW * 512) * sizeof(float2);
+  const int grid = (int)std::min<int64_t>(Q.total_runs, (int64_t)ctx->num_sms * (16 / NW));
+  void (*k)(const Istft32Params) = Q.hop == 32 ? istft512_tile_kernel<true> : istft512_tile_kernel<false>;
+  SSQ_CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k<<<grid, NW * 32, smem, ctx->stream>>>(Q);
+  SSQ_TRY(ssq_check_launch(ctx, "istft512_tile_kernel"));
+  ctx->last_kernel = "istft512_tile_kernel";
+  return SSQ_OK;
 }

@@ -12,10 +12,11 @@
 #define I1K_AS 514  // tile row stride (float2): 2 AS = 4 mod 32 -> the transposed load (8 frames x 4 rows per warp step) is
                     // bank-conflict free; 1028 floats >= 1024 samples
 
-template <int NW>  // F = 2 NW frames per tile
-__global__ void __launch_bounds__(NW * 32, 3) istft1024_tile_kernel(const Istft32Params P) {
-  constexpr int N = 1024, AS = I1K_AS, XS = R1K_XS, F = 2 * NW;
-  constexpr bool PK = SSQ_PK_DEFAULT;
+#define I1K_NW 4    // warps per CTA; F = 2 NW frames per tile
+
+__global__ void __launch_bounds__(I1K_NW * 32, 3) istft1024_tile_kernel(const Istft32Params P) {
+  constexpr int N = 1024, AS = I1K_AS, XS = R1K_XS, NW = I1K_NW, F = 2 * NW;
+  constexpr bool PK = true;
   static_assert(NW == 4, "the load mapping below assumes 4 warps x 8 frames");
   extern __shared__ float2 smem[];
   float2* S = smem;  // [F][AS]
@@ -127,4 +128,23 @@ __global__ void __launch_bounds__(NW * 32, 3) istft1024_tile_kernel(const Istft3
     }
     __syncthreads();
   }
+}
+
+static ssq_status istft1024_launch(ssq_ctx* ctx, Istft32Params& Q, bool* done) {
+  *done = false;
+  if (Q.n_fft != 1024 || ctx->opt.no_r1024) return SSQ_OK;
+  constexpr int NW = I1K_NW, F = 2 * NW;
+  Q.run = F;
+  Q.runs_per_channel = (Q.n_use + F - 1) / F;
+  Q.total_runs = Q.runs_per_channel * Q.channels;
+  // 32-bit tile indices; the tile span inside the range of ssq_fast_div
+  if (Q.total_runs > (int64_t)0x7ff00000 || (int64_t)(F - 1) * Q.hop + 1024 >= ((int64_t)1 << 22)) return SSQ_OK;
+  *done = true;
+  const size_t smem = ((size_t)F * I1K_AS + (size_t)NW * 32 * R1K_XS) * sizeof(float2);
+  const int grid = (int)std::min<int64_t>(Q.total_runs, (int64_t)ctx->num_sms * 3);
+  SSQ_CUDA_TRY(ctx, cudaFuncSetAttribute(istft1024_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  istft1024_tile_kernel<<<grid, NW * 32, smem, ctx->stream>>>(Q);
+  SSQ_TRY(ssq_check_launch(ctx, "istft1024_tile_kernel"));
+  ctx->last_kernel = "istft1024_tile_kernel";
+  return SSQ_OK;
 }

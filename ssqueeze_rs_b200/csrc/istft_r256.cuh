@@ -8,11 +8,11 @@
 #include "stft_r256.cuh"
 
 #define I256_AS 131  // tile row stride (float2): odd; 262 floats >= 256 samples
+#define I256_NW 4    // warps per CTA; F = 8 NW frames per tile
 
-template <int NW>  // F = 8 NW frames per tile
-__global__ void __launch_bounds__(NW * 32, 3) istft256_tile_kernel(const Istft32Params P) {
-  constexpr int N = 256, AS = I256_AS, XS = R1K_XS, F = 8 * NW;
-  constexpr bool PK = SSQ_PK_DEFAULT;
+__global__ void __launch_bounds__(I256_NW * 32, 3) istft256_tile_kernel(const Istft32Params P) {
+  constexpr int N = 256, AS = I256_AS, XS = R1K_XS, NW = I256_NW, F = 8 * NW;
+  constexpr bool PK = true;
   static_assert(NW == 4, "the load mapping below assumes 4 warps x 32 frames");
   extern __shared__ float2 smem[];
   float2* S = smem;  // [F][AS]
@@ -137,4 +137,23 @@ __global__ void __launch_bounds__(NW * 32, 3) istft256_tile_kernel(const Istft32
     }
     __syncthreads();
   }
+}
+
+static ssq_status istft256_launch(ssq_ctx* ctx, Istft32Params& Q, bool* done) {
+  *done = false;
+  if (Q.n_fft != 256 || ctx->opt.no_r256) return SSQ_OK;
+  constexpr int NW = I256_NW, F = 8 * NW;
+  Q.run = F;
+  Q.runs_per_channel = (Q.n_use + F - 1) / F;
+  Q.total_runs = Q.runs_per_channel * Q.channels;
+  // 32-bit tile indices; the tile span inside the range of ssq_fast_div
+  if (Q.total_runs > (int64_t)0x7ff00000 || (int64_t)(F - 1) * Q.hop + 256 >= ((int64_t)1 << 22)) return SSQ_OK;
+  *done = true;
+  const size_t smem = ((size_t)F * I256_AS + (size_t)NW * 32 * R1K_XS) * sizeof(float2);
+  const int grid = (int)std::min<int64_t>(Q.total_runs, (int64_t)ctx->num_sms * 3);
+  SSQ_CUDA_TRY(ctx, cudaFuncSetAttribute(istft256_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  istft256_tile_kernel<<<grid, NW * 32, smem, ctx->stream>>>(Q);
+  SSQ_TRY(ssq_check_launch(ctx, "istft256_tile_kernel"));
+  ctx->last_kernel = "istft256_tile_kernel";
+  return SSQ_OK;
 }

@@ -49,12 +49,11 @@ struct ssq_ctx {
   // pinned staging of the float64 entry points (two chunks: copy of chunk i+1 overlaps the conversion of chunk i)
   void* pin[2] = {nullptr, nullptr};
   cudaEvent_t pin_ev[2] = {nullptr, nullptr};
-  // kernel-selection switches (measurement and cross-checks only, DESIGN 6c): seeded once from the
-  // environment (SSQ_<NAME>) by ssq_ctx_create, changed with ssq_ctx_set_option
+  // context options (DESIGN 6c), set only through ssq_ctx_set_option.  The first four select the reference paths
+  // the tests check the fast kernels against: the generic shared-memory STFT kernels for n_fft 512 / 1024 / 256,
+  // and the ordered, bit-deterministic ssq_cwt tail
   struct Options {
-    int no_h32r = 0, h32r_nw = 0, no_r1024 = 0, no_r256 = 0, istft_nw = 8;
-    int no_fft128 = 0, fft128_tc = 0, no_cwt_prune = 0, no_cwt_fused = 0, cwt_fused_tc = 32;
-    int64_t cwt_ws_mb = 0;
+    int no_h32r = 0, no_r1024 = 0, no_r256 = 0, no_cwt_fused = 0;
     // STFT family framed as upstream ssqueezepy frames it (left pad n_fft / 2, the larger side for even n_fft:
     // old/ssqueezepy/utils/common.py:116-120) instead of the crate's (n_fft - 1) / 2 (stft_utils.rs:22); this one
     // does change results -- it is the switch of the upstream-compatible mode (ssqueeze_rs_b200/compat.py)
@@ -137,12 +136,7 @@ __device__ __forceinline__ float2 up2(ssq_u64 v) {
 // PK = false selects the scalar forms: the packed ones need aligned register pairs, and a kernel
 // that already sits at its register cap can lose more to the spills than it gains (the stft mode
 // of the n_fft = 512 kernel: 18.5 ms packed with 56 B of spills, 16.8 ms scalar on 384 channels).
-#ifdef SSQ_SCALAR_COMPLEX  // A/B switch for measurements
-#define SSQ_PK_DEFAULT false
-#else
-#define SSQ_PK_DEFAULT true
-#endif
-template <bool PK = SSQ_PK_DEFAULT>
+template <bool PK = true>
 __device__ __forceinline__ float2 add2(float2 a, float2 b) {
   if constexpr (PK) {
     ssq_u64 r;
@@ -152,7 +146,7 @@ __device__ __forceinline__ float2 add2(float2 a, float2 b) {
     return make_float2(a.x + b.x, a.y + b.y);
   }
 }
-template <bool PK = SSQ_PK_DEFAULT>
+template <bool PK = true>
 __device__ __forceinline__ float2 sub2(float2 a, float2 b) {
   if constexpr (PK) {
     ssq_u64 r;
@@ -162,7 +156,7 @@ __device__ __forceinline__ float2 sub2(float2 a, float2 b) {
     return make_float2(a.x - b.x, a.y - b.y);
   }
 }
-template <bool PK = SSQ_PK_DEFAULT>
+template <bool PK = true>
 __device__ __forceinline__ float2 mul2(float2 a, float2 b) {
   if constexpr (PK) {
     ssq_u64 r;
@@ -172,7 +166,7 @@ __device__ __forceinline__ float2 mul2(float2 a, float2 b) {
     return make_float2(a.x * b.x, a.y * b.y);
   }
 }
-template <bool PK = SSQ_PK_DEFAULT>
+template <bool PK = true>
 __device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c) {
   if constexpr (PK) {
     ssq_u64 r;
@@ -183,17 +177,17 @@ __device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c) {
   }
 }
 __device__ __forceinline__ float2 bc2(float s) { return make_float2(s, s); }
-template <bool PK = SSQ_PK_DEFAULT>
+template <bool PK = true>
 __device__ __forceinline__ float2 cmulf(float2 a, float2 b) {  // (a.x b.x - a.y b.y, a.y b.x + a.x b.y)
   return fma2<PK>(make_float2(a.y, a.x), make_float2(-b.y, b.y), mul2<PK>(a, bc2(b.x)));
 }
-template <bool PK = SSQ_PK_DEFAULT>
+template <bool PK = true>
 __device__ __forceinline__ float2 cmulcf(float2 a, float2 b) {  // a * conj(b)
   return fma2<PK>(make_float2(a.y, a.x), make_float2(b.y, -b.y), mul2<PK>(a, bc2(b.x)));
 }
-template <bool PK = SSQ_PK_DEFAULT>
+template <bool PK = true>
 __device__ __forceinline__ float2 caddf(float2 a, float2 b) { return add2<PK>(a, b); }
-template <bool PK = SSQ_PK_DEFAULT>
+template <bool PK = true>
 __device__ __forceinline__ float2 csubf(float2 a, float2 b) { return sub2<PK>(a, b); }
 __device__ __forceinline__ float2 cmi(float2 a) { return make_float2(a.y, -a.x); }  // a * (-i)
 __device__ __forceinline__ float2 cpi(float2 a) { return make_float2(-a.y, a.x); }  // a * (+i)

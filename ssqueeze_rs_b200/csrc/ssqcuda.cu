@@ -77,14 +77,6 @@ extern "C" ssq_status ssq_ctx_create(int device, ssq_ctx** out) {
     return ssq_fail(nullptr, SSQ_ECUDA, "stream/event creation: %s", cudaGetErrorString(e));
   }
   c->stream = c->own_stream;
-  // switches: read from the environment once, here (never on the launch path)
-  static const char* const names[] = {"no_h32r", "h32r_nw", "no_r1024", "no_r256", "istft_nw", "no_fft128",
-                                      "fft128_tc", "no_cwt_prune", "no_cwt_fused", "cwt_fused_tc", "cwt_ws_mb", "upstream_framing"};
-  for (const char* nm : names) {
-    std::string env = "SSQ_";
-    for (const char* q = nm; *q; ++q) env += (char)toupper((unsigned char)*q);
-    if (const char* v = getenv(env.c_str())) (void)ssq_ctx_set_option(c, nm, atoll(v));
-  }
   *out = c;
   return SSQ_OK;
 }
@@ -94,16 +86,9 @@ extern "C" ssq_status ssq_ctx_set_option(ssq_ctx* ctx, const char* name, int64_t
   const std::string n(name);
   ssq_ctx::Options& o = ctx->opt;
   if (n == "no_h32r") o.no_h32r = value != 0;
-  else if (n == "h32r_nw") o.h32r_nw = (value == 4 || value == 8) ? (int)value : 0;
   else if (n == "no_r1024") o.no_r1024 = value != 0;
   else if (n == "no_r256") o.no_r256 = value != 0;
-  else if (n == "istft_nw") o.istft_nw = value == 4 ? 4 : 8;
-  else if (n == "no_fft128") o.no_fft128 = value != 0;
-  else if (n == "fft128_tc") o.fft128_tc = (value == 16 || value == 32 || value == 64) ? (int)value : 0;
-  else if (n == "no_cwt_prune") o.no_cwt_prune = value != 0;
   else if (n == "no_cwt_fused") o.no_cwt_fused = value != 0;
-  else if (n == "cwt_fused_tc") o.cwt_fused_tc = value == 32 ? 32 : 64;
-  else if (n == "cwt_ws_mb") o.cwt_ws_mb = value > 0 ? value : 0;
   else if (n == "upstream_framing") o.upstream_framing = value != 0;
   else return ssq_fail(ctx, SSQ_EINVAL, "ssq_ctx_set_option: unknown option '%s'", name);
   return SSQ_OK;
@@ -453,18 +438,11 @@ static ssq_status run_stft_family(ssq_ctx* ctx, const StftCall& c) {
 
   SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
   bool done = false;
-  {  // diagnostic outputs (aux_*) do not change the kernel selection: the register kernels carry them as a
-     // compile-time variant of the same code
-    ssq_status st = stft_h32r_launch(ctx, P, &done);
-    if (st != SSQ_OK) return st;
-    if (!done) {
-      st = stft_r1024_launch(ctx, P, &done);
-      if (st != SSQ_OK) return st;
-    }
-    if (!done) {
-      st = stft_r256_launch(ctx, P, &done);
-      if (st != SSQ_OK) return st;
-    }
+  // diagnostic outputs (aux_*) do not change the kernel selection: the register kernels carry them as a
+  // compile-time variant of the same code
+  for (auto launch : {stft_h32r_launch, stft_r1024_launch, stft_r256_launch}) {
+    SSQ_TRY(launch(ctx, P, &done));
+    if (done) break;
   }
   if (!done) SSQ_TRY(stft_rows_run(ctx, P, &done));  // n_fft > 4096, or not a power of two: batched row FFTs
   if (!done) {
@@ -583,153 +561,54 @@ extern "C" ssq_status ssq_istft_batch_f32(ssq_ctx* ctx, const float* d_Sx, int64
   SSQ_TRY(devbuf_reserve(ctx, ctx->ws_misc, (size_t)channels * L * sizeof(float)));
   SSQ_CUDA_TRY(ctx, cudaMemsetAsync(ctx->ws_misc.p, 0, (size_t)channels * L * sizeof(float), ctx->stream));
 
-  if (n_fft == 512 && !ctx->opt.no_h32r &&
-      (int64_t)31 * hop + 512 < ((int64_t)1 << 22)) {  // tile span inside the range of ssq_fast_div
-    Istft32Params Q;
-    memset(&Q, 0, sizeof(Q));
-    Q.Sx = (const float2*)d_Sx;
-    Q.channels = (int)channels;
-    Q.n_frames = n_frames;
-    Q.n_use = std::min<int64_t>(n_frames, max_hops);
-    Q.L = L;
-    Q.wa = T.wa;
-    Q.tw = T.tw;
-    Q.xacc = (float*)ctx->ws_misc.p;
-    Q.hop = hop;
-    SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    {
-      // 8-warp CTAs / 32-frame tiles (SSQ_ISTFT_NW=4: 4 warps / 16 frames, 4 CTAs per SM -- measured 10.2 vs 9.5 ms)
-      const int nw = ctx->opt.istft_nw;
-      const int F = nw == 8 ? 32 : 16, NWc = nw == 8 ? 8 : 4;
-      Q.run = F;
-      Q.runs_per_channel = (Q.n_use + F - 1) / F;
-      Q.total_runs = Q.runs_per_channel * channels;
-      const size_t smem = ((size_t)72 + (size_t)F * I32T_AS + (size_t)NWc * 512) * sizeof(float2);
-      const int grid = (int)std::min<int64_t>(Q.total_runs, (int64_t)ctx->num_sms * (16 / NWc));
-      void (*k)(const Istft32Params) = NWc == 8 ? (hop == 32 ? istft512_tile_kernel<true, 8> : istft512_tile_kernel<false, 8>)
-                                                : (hop == 32 ? istft512_tile_kernel<true, 4> : istft512_tile_kernel<false, 4>);
-      SSQ_CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k<<<grid, NWc * 32, smem, ctx->stream>>>(Q);
-      SSQ_TRY(ssq_check_launch(ctx, "istft512_tile_kernel"));
-      ctx->last_kernel = "istft512_tile_kernel";
-    }
-    SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-    ctx->ev_valid = true;
-    dim3 g((unsigned)((n_out + ISTFT_FIN_PER_BLOCK - 1) / ISTFT_FIN_PER_BLOCK), (unsigned)channels);
-    istft_finalize_kernel<<<g, 256, 0, ctx->stream>>>((const float*)ctx->ws_misc.p, L, n_out, n_fft, hop,
-                                                      istft_left(ctx, n_fft), max_hops, T.wpow, d_xout);
-    SSQ_TRY(ssq_check_launch(ctx, "istft_finalize_kernel"));
-    return SSQ_OK;
-  }
-
-  if (n_fft == 256 && !ctx->opt.no_r256) {
-    Istft32Params Q;
-    memset(&Q, 0, sizeof(Q));
-    Q.Sx = (const float2*)d_Sx;
-    Q.channels = (int)channels;
-    Q.n_frames = n_frames;
-    Q.n_use = std::min<int64_t>(n_frames, max_hops);
-    Q.L = L;
-    Q.wa = T.wa;
-    Q.tw = T.tw;
-    Q.xacc = (float*)ctx->ws_misc.p;
-    Q.hop = hop;
-    constexpr int NW = 4, F = 32;
-    Q.run = F;
-    Q.runs_per_channel = (Q.n_use + F - 1) / F;
-    Q.total_runs = Q.runs_per_channel * channels;
-    if (Q.total_runs <= (int64_t)0x7ff00000 && (int64_t)(F - 1) * hop + 256 < ((int64_t)1 << 22)) {
-      const size_t smem = ((size_t)F * I256_AS + (size_t)NW * 32 * R1K_XS) * sizeof(float2);
-      const int grid = (int)std::min<int64_t>(Q.total_runs, (int64_t)ctx->num_sms * 3);
-      SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-      SSQ_CUDA_TRY(ctx, cudaFuncSetAttribute(istft256_tile_kernel<NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      istft256_tile_kernel<NW><<<grid, NW * 32, smem, ctx->stream>>>(Q);
-      SSQ_TRY(ssq_check_launch(ctx, "istft256_tile_kernel"));
-      ctx->last_kernel = "istft256_tile_kernel";
-      SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-      ctx->ev_valid = true;
-      dim3 g((unsigned)((n_out + ISTFT_FIN_PER_BLOCK - 1) / ISTFT_FIN_PER_BLOCK), (unsigned)channels);
-      istft_finalize_kernel<<<g, 256, 0, ctx->stream>>>((const float*)ctx->ws_misc.p, L, n_out, n_fft, hop,
-                                                        istft_left(ctx, n_fft), max_hops, T.wpow, d_xout);
-      SSQ_TRY(ssq_check_launch(ctx, "istft_finalize_kernel"));
-      return SSQ_OK;
-    }
-  }
-
-  if (n_fft == 1024 && !ctx->opt.no_r1024) {
-    Istft32Params Q;
-    memset(&Q, 0, sizeof(Q));
-    Q.Sx = (const float2*)d_Sx;
-    Q.channels = (int)channels;
-    Q.n_frames = n_frames;
-    Q.n_use = std::min<int64_t>(n_frames, max_hops);
-    Q.L = L;
-    Q.wa = T.wa;
-    Q.tw = T.tw;
-    Q.xacc = (float*)ctx->ws_misc.p;
-    Q.hop = hop;
-    constexpr int NW = 4, F = 8;
-    Q.run = F;
-    Q.runs_per_channel = (Q.n_use + F - 1) / F;
-    Q.total_runs = Q.runs_per_channel * channels;
-    if (Q.total_runs <= (int64_t)0x7ff00000 && (int64_t)(F - 1) * hop + 1024 < ((int64_t)1 << 22)) {
-      const size_t smem = ((size_t)F * I1K_AS + (size_t)NW * 32 * R1K_XS) * sizeof(float2);
-      const int grid = (int)std::min<int64_t>(Q.total_runs, (int64_t)ctx->num_sms * 3);
-      SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-      SSQ_CUDA_TRY(ctx, cudaFuncSetAttribute(istft1024_tile_kernel<NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      istft1024_tile_kernel<NW><<<grid, NW * 32, smem, ctx->stream>>>(Q);
-      SSQ_TRY(ssq_check_launch(ctx, "istft1024_tile_kernel"));
-      ctx->last_kernel = "istft1024_tile_kernel";
-      SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-      ctx->ev_valid = true;
-      dim3 g((unsigned)((n_out + ISTFT_FIN_PER_BLOCK - 1) / ISTFT_FIN_PER_BLOCK), (unsigned)channels);
-      istft_finalize_kernel<<<g, 256, 0, ctx->stream>>>((const float*)ctx->ws_misc.p, L, n_out, n_fft, hop,
-                                                        istft_left(ctx, n_fft), max_hops, T.wpow, d_xout);
-      SSQ_TRY(ssq_check_launch(ctx, "istft_finalize_kernel"));
-      return SSQ_OK;
-    }
-  }
-
-  IstftParams P;
-  memset(&P, 0, sizeof(P));
-  P.Sx = (const float2*)d_Sx;
-  P.channels = (int)channels;
-  P.n_fft = n_fft;
-  P.hop = hop;
-  P.n_freqs = (int)n_freqs;
-  P.log2n = ilog2_exact(n_fft);
-  P.is_pow2 = P.log2n >= 0;
-  P.n_frames = n_frames;
-  P.n_use = std::min<int64_t>(n_frames, max_hops);
-  P.L = L;
-  P.wa = T.wa;
-  P.tw = T.tw;
-  P.xacc = (float*)ctx->ws_misc.p;
-  {  // n_fft > 4096 or not a power of two: batched row FFTs
-    bool rows_done = false;
-    SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-    SSQ_TRY(istft_rows_run(ctx, P, &rows_done));
-    if (rows_done) {
-      SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-      ctx->ev_valid = true;
-      dim3 g((unsigned)((n_out + ISTFT_FIN_PER_BLOCK - 1) / ISTFT_FIN_PER_BLOCK), (unsigned)channels);
-      istft_finalize_kernel<<<g, 256, 0, ctx->stream>>>((const float*)ctx->ws_misc.p, L, n_out, n_fft, hop,
-                                                        istft_left(ctx, n_fft), max_hops, T.wpow, d_xout);
-      SSQ_TRY(ssq_check_launch(ctx, "istft_finalize_kernel"));
-      return SSQ_OK;
-    }
-  }
-  TilePlan tp;
-  SSQ_TRY(plan_generic_tiles(ctx, n_fft, (int)n_freqs, P.n_use, (int)channels, &tp, &P.tiles_per_channel,
-                             &P.total_tiles));
-  P.F = tp.F;
-  P.acc_stride = tp.acc_stride;
+  Istft32Params Q;
+  memset(&Q, 0, sizeof(Q));
+  Q.Sx = (const float2*)d_Sx;
+  Q.channels = (int)channels;
+  Q.n_frames = n_frames;
+  Q.n_use = std::min<int64_t>(n_frames, max_hops);
+  Q.L = L;
+  Q.wa = T.wa;
+  Q.tw = T.tw;
+  Q.xacc = (float*)ctx->ws_misc.p;
+  Q.hop = hop;
+  Q.n_fft = n_fft;
   SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
-  SSQ_CUDA_TRY(ctx,
-               cudaFuncSetAttribute(istft_ola_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem));
-  istft_ola_kernel<<<tp.grid, tp.nw * 32, tp.smem, ctx->stream>>>(P);
-  SSQ_TRY(ssq_check_launch(ctx, "istft_ola_kernel"));
-  ctx->last_kernel = "istft_ola_kernel";
+  bool done = false;
+  for (auto launch : {istft512_launch, istft256_launch, istft1024_launch}) {
+    SSQ_TRY(launch(ctx, Q, &done));
+    if (done) break;
+  }
+  if (!done) {
+    IstftParams P;
+    memset(&P, 0, sizeof(P));
+    P.Sx = Q.Sx;
+    P.channels = Q.channels;
+    P.n_fft = n_fft;
+    P.hop = hop;
+    P.n_freqs = (int)n_freqs;
+    P.log2n = ilog2_exact(n_fft);
+    P.is_pow2 = P.log2n >= 0;
+    P.n_frames = n_frames;
+    P.n_use = Q.n_use;
+    P.L = L;
+    P.wa = T.wa;
+    P.tw = T.tw;
+    P.xacc = Q.xacc;
+    SSQ_TRY(istft_rows_run(ctx, P, &done));  // n_fft > 4096, or not a power of two: batched row FFTs
+    if (!done) {
+      TilePlan tp;
+      SSQ_TRY(plan_generic_tiles(ctx, n_fft, (int)n_freqs, P.n_use, (int)channels, &tp, &P.tiles_per_channel,
+                                 &P.total_tiles));
+      P.F = tp.F;
+      P.acc_stride = tp.acc_stride;
+      SSQ_CUDA_TRY(ctx,
+                   cudaFuncSetAttribute(istft_ola_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem));
+      istft_ola_kernel<<<tp.grid, tp.nw * 32, tp.smem, ctx->stream>>>(P);
+      SSQ_TRY(ssq_check_launch(ctx, "istft_ola_kernel"));
+      ctx->last_kernel = "istft_ola_kernel";
+    }
+  }
   SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
   ctx->ev_valid = true;
   dim3 g((unsigned)((n_out + ISTFT_FIN_PER_BLOCK - 1) / ISTFT_FIN_PER_BLOCK), (unsigned)channels);

@@ -220,13 +220,16 @@ __device__ __noinline__ float h32r_edge_sample(const float* x, int64_t n, int64_
   return stft_sample(x, n, p, left, padtype, origin);
 }
 
-// NW warps per CTA (8: 32-frame tile, 2 CTAs per SM; 4: 16-frame tile, 4 CTAs per SM -- the same 16
-// warps per SM, half the barrier domain).
+// Warps per CTA, 16 per SM either way.  4 for ssq_stft (16-frame tiles, 128 B row segments, 4 CTAs per SM: half the
+// barrier domain of the 8-warp shape, which was 3.6 % slower); 8 for the faster stft mode, which writes at > 2.5 TB/s
+// and needs the 256 B segments of 32-frame tiles at full scale (384 channels: 18.1 vs 26.5 ms).
+#define H32R_NW(MODE) ((MODE) == 1 ? 8 : 4)
+
 // SLIDE: hop == 32, the register sliding window (one new sample per lane and frame).  Otherwise any hop:
 // the 16 samples of every frame are (re)loaded, still a whole frame ahead of their use.
-template <int MODE, int SQZ, int NW, bool SLIDE, bool DBG = false>
-__global__ void __launch_bounds__(NW * 32, 16 / NW) ssq_stft512_h32r_kernel(const StftParams P) {
-  constexpr int N = 512, AS = H32R_AS, F = 4 * NW;
+template <int MODE, int SQZ, bool SLIDE, bool DBG = false>
+__global__ void __launch_bounds__(H32R_NW(MODE) * 32, 16 / H32R_NW(MODE)) ssq_stft512_h32r_kernel(const StftParams P) {
+  constexpr int N = 512, AS = H32R_AS, NW = H32R_NW(MODE), F = 4 * NW;
   // stft at hop 32: two frames per FFT (z = x_A w + i x_B w; frame B's samples are frame A's window
   // shifted by one position), so a warp runs 2 FFTs for its 4 frames
   constexpr bool PAIR = (MODE == 1) && SLIDE;
@@ -396,9 +399,10 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) ssq_stft512_h32r_kernel(cons
   }
 }
 
-template <int NW>
-static ssq_status stft_h32r_launch_nw(ssq_ctx* ctx, StftParams& P, bool* done) {
-  constexpr int F = 4 * NW;
+static ssq_status stft_h32r_launch(ssq_ctx* ctx, StftParams& P, bool* done) {
+  *done = false;
+  if (P.n_fft != 512 || ctx->opt.no_h32r) return SSQ_OK;
+  const int NW = H32R_NW(P.mode), F = 4 * NW;
   P.F = F;
   P.acc_stride = H32R_AS;
   P.tiles_per_channel = (P.n_frames + F - 1) / F;
@@ -411,31 +415,20 @@ static ssq_status stft_h32r_launch_nw(ssq_ctx* ctx, StftParams& P, bool* done) {
   void (*k)(const StftParams);
   const bool dbg = P.mode == 0 && (P.aux_Sx || P.aux_dSx || P.aux_w || P.aux_kb);
   if (dbg)  // the same kernel with the diagnostic stores compiled in (parity tests)
-    k = P.hop == 32 ? (leb ? ssq_stft512_h32r_kernel<0, 1, NW, true, true> : ssq_stft512_h32r_kernel<0, 0, NW, true, true>)
-                    : (leb ? ssq_stft512_h32r_kernel<0, 1, NW, false, true> : ssq_stft512_h32r_kernel<0, 0, NW, false, true>);
+    k = P.hop == 32 ? (leb ? ssq_stft512_h32r_kernel<0, 1, true, true> : ssq_stft512_h32r_kernel<0, 0, true, true>)
+                    : (leb ? ssq_stft512_h32r_kernel<0, 1, false, true> : ssq_stft512_h32r_kernel<0, 0, false, true>);
   else if (P.hop == 32)
-    k = P.mode == 1 ? ssq_stft512_h32r_kernel<1, 0, NW, true>
-        : leb       ? ssq_stft512_h32r_kernel<0, 1, NW, true>
-                    : ssq_stft512_h32r_kernel<0, 0, NW, true>;
+    k = P.mode == 1 ? ssq_stft512_h32r_kernel<1, 0, true>
+        : leb       ? ssq_stft512_h32r_kernel<0, 1, true>
+                    : ssq_stft512_h32r_kernel<0, 0, true>;
   else
-    k = P.mode == 1 ? ssq_stft512_h32r_kernel<1, 0, NW, false>
-        : leb       ? ssq_stft512_h32r_kernel<0, 1, NW, false>
-                    : ssq_stft512_h32r_kernel<0, 0, NW, false>;
+    k = P.mode == 1 ? ssq_stft512_h32r_kernel<1, 0, false>
+        : leb       ? ssq_stft512_h32r_kernel<0, 1, false>
+                    : ssq_stft512_h32r_kernel<0, 0, false>;
   SSQ_CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k<<<grid, NW * 32, smem, ctx->stream>>>(P);
   const char* name = P.mode == 1 ? "ssq_stft512_h32r_kernel<stft>" : "ssq_stft512_h32r_kernel<ssq>";
   SSQ_TRY(ssq_check_launch(ctx, name));
   ctx->last_kernel = name;
-  return SSQ_OK;
-}
-
-static ssq_status stft_h32r_launch(ssq_ctx* ctx, StftParams& P, bool* done) {
-  *done = false;
-  if (P.n_fft != 512 || ctx->opt.no_h32r) return SSQ_OK;
-  // 4-warp CTAs (16-frame tiles, 128 B row segments) win for ssq_stft; the faster stft mode writes at
-  // > 2.5 TB/s and needs the 256 B segments of the 8-warp shape at full scale (384 channels: 18.1 vs 26.5 ms)
-  const int nw_env = ctx->opt.h32r_nw ? ctx->opt.h32r_nw : (P.mode == 1 ? 8 : 4);
-  if (nw_env == 4) SSQ_TRY(stft_h32r_launch_nw<4>(ctx, P, done));
-  else SSQ_TRY(stft_h32r_launch_nw<8>(ctx, P, done));
   return SSQ_OK;
 }

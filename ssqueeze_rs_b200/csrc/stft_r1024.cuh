@@ -152,11 +152,13 @@ __device__ __noinline__ void r1k_collision(float2* col, unsigned* T, int kb, flo
 }
 
 
-// NW warps per CTA, F frames per tile (F / NW per warp).
-template <int MODE, int SQZ, int NW, int F, bool DBG = false>
-__global__ void __launch_bounds__(NW * 32, 3) ssq_stft1024_kernel(const StftParams P) {
-  constexpr int N = 1024, AS = R1K_AS, XS = R1K_XS, FPW = F / NW;
-  constexpr bool PK = SSQ_PK_DEFAULT;
+#define R1K_NW 4  // warps per CTA
+#define R1K_F 8   // frames per tile (F / NW per warp)
+
+template <int MODE, int SQZ, bool DBG = false>
+__global__ void __launch_bounds__(R1K_NW * 32, 3) ssq_stft1024_kernel(const StftParams P) {
+  constexpr int N = 1024, AS = R1K_AS, XS = R1K_XS, NW = R1K_NW, F = R1K_F, FPW = F / NW;
+  constexpr bool PK = true;
   static_assert(F % NW == 0 && (F / NW) % 2 == 0, "frames per warp: even (stft mode packs pairs)");
   extern __shared__ float2 smem[];
   float2* acc = smem;  // [F][AS]
@@ -346,7 +348,7 @@ __global__ void __launch_bounds__(NW * 32, 3) ssq_stft1024_kernel(const StftPara
 static ssq_status stft_r1024_launch(ssq_ctx* ctx, StftParams& P, bool* done) {
   *done = false;
   if (P.n_fft != 1024 || ctx->opt.no_r1024) return SSQ_OK;
-  constexpr int NW = 4, F = 8;
+  constexpr int NW = R1K_NW, F = R1K_F;
   StftParams Q = P;
   Q.F = F;
   Q.acc_stride = R1K_AS;
@@ -358,10 +360,10 @@ static ssq_status stft_r1024_launch(ssq_ctx* ctx, StftParams& P, bool* done) {
   const int grid = (int)std::min<int64_t>(Q.total_tiles, (int64_t)ctx->num_sms * 3);
   const bool leb = P.squeezing == SSQ_SQUEEZE_LEBESGUE;
   const bool dbg = P.mode == 0 && (P.aux_Sx || P.aux_dSx || P.aux_w || P.aux_kb);
-  void (*k)(const StftParams) = P.mode == 1 ? ssq_stft1024_kernel<1, 0, NW, F>
-                                : dbg       ? (leb ? ssq_stft1024_kernel<0, 1, NW, F, true> : ssq_stft1024_kernel<0, 0, NW, F, true>)
-                                : leb       ? ssq_stft1024_kernel<0, 1, NW, F>
-                                            : ssq_stft1024_kernel<0, 0, NW, F>;
+  void (*k)(const StftParams) = P.mode == 1 ? ssq_stft1024_kernel<1, 0>
+                                : dbg       ? (leb ? ssq_stft1024_kernel<0, 1, true> : ssq_stft1024_kernel<0, 0, true>)
+                                : leb       ? ssq_stft1024_kernel<0, 1>
+                                            : ssq_stft1024_kernel<0, 0>;
   SSQ_CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k<<<grid, NW * 32, smem, ctx->stream>>>(Q);
   const char* name = P.mode == 1 ? "ssq_stft1024_kernel<stft>" : "ssq_stft1024_kernel<ssq>";

@@ -54,11 +54,13 @@ __device__ __noinline__ void r256_collision(float2* col, unsigned short* T, int 
   }
 }
 
-// NW warps per CTA, F frames per tile (groups of four per warp).
-template <int MODE, int SQZ, int NW, int F, bool DBG = false>
-__global__ void __launch_bounds__(NW * 32, MODE == 0 ? 4 : 3) ssq_stft256_kernel(const StftParams P) {
-  constexpr int N = 256, AS = R256_AS, XS = R1K_XS, SS = R256_SS, GPW = F / (4 * NW);
-  constexpr bool PK = SSQ_PK_DEFAULT;
+#define R256_NW 4  // warps per CTA
+
+// F frames per tile (groups of four per warp).
+template <int MODE, int SQZ, int F, bool DBG = false>
+__global__ void __launch_bounds__(R256_NW * 32, MODE == 0 ? 4 : 3) ssq_stft256_kernel(const StftParams P) {
+  constexpr int N = 256, AS = R256_AS, XS = R1K_XS, SS = R256_SS, NW = R256_NW, GPW = F / (4 * NW);
+  constexpr bool PK = true;
   static_assert(F % (4 * NW) == 0, "a warp takes its frames four at a time");
   // stft mode: two groups per FFT (z = x_A w + i x_B w, frame B = frame A + 4)
   constexpr int STEP = (MODE == 1) ? 2 : 1;
@@ -272,8 +274,9 @@ __global__ void __launch_bounds__(NW * 32, MODE == 0 ? 4 : 3) ssq_stft256_kernel
   }
 }
 
-template <int NW, int F>
+template <int F>
 static ssq_status stft_r256_launch_f(ssq_ctx* ctx, StftParams& P, bool* done) {
+  constexpr int NW = R256_NW;
   StftParams Q = P;
   Q.F = F;
   Q.acc_stride = R256_AS;
@@ -285,10 +288,10 @@ static ssq_status stft_r256_launch_f(ssq_ctx* ctx, StftParams& P, bool* done) {
   const int grid = (int)std::min<int64_t>(Q.total_tiles, (int64_t)ctx->num_sms * (F == 32 ? 3 : 4));
   const bool leb = P.squeezing == SSQ_SQUEEZE_LEBESGUE;
   void (*k)(const StftParams);
-  if constexpr (F == 32) k = ssq_stft256_kernel<1, 0, NW, F>;
+  if constexpr (F == 32) k = ssq_stft256_kernel<1, 0, F>;
   else if (P.aux_Sx || P.aux_dSx || P.aux_w || P.aux_kb)
-    k = leb ? ssq_stft256_kernel<0, 1, NW, F, true> : ssq_stft256_kernel<0, 0, NW, F, true>;
-  else k = leb ? ssq_stft256_kernel<0, 1, NW, F> : ssq_stft256_kernel<0, 0, NW, F>;
+    k = leb ? ssq_stft256_kernel<0, 1, F, true> : ssq_stft256_kernel<0, 0, F, true>;
+  else k = leb ? ssq_stft256_kernel<0, 1, F> : ssq_stft256_kernel<0, 0, F>;
   SSQ_CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k<<<grid, NW * 32, smem, ctx->stream>>>(Q);
   const char* name = P.mode == 1 ? "ssq_stft256_kernel<stft>" : "ssq_stft256_kernel<ssq>";
@@ -302,5 +305,5 @@ static ssq_status stft_r256_launch(ssq_ctx* ctx, StftParams& P, bool* done) {
   *done = false;
   if (P.n_fft != 256 || ctx->opt.no_r256) return SSQ_OK;
   // ssq: 16-frame tiles (one group of four frames per warp); stft: 32-frame tiles, two groups per FFT
-  return P.mode == 1 ? stft_r256_launch_f<4, 32>(ctx, P, done) : stft_r256_launch_f<4, 16>(ctx, P, done);
+  return P.mode == 1 ? stft_r256_launch_f<32>(ctx, P, done) : stft_r256_launch_f<16>(ctx, P, done);
 }

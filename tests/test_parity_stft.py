@@ -591,6 +591,28 @@ def test_fast_kernels_agree_and_are_deterministic():
     assert float((outs["h32r"][0].sum(dim=1) - ref.sum(dim=1)).abs().max()) < 2e-3 * sc
 
 
+def test_context_options_are_set_only_through_set_option(monkeypatch):
+    """The context has five options; the names of the removed CTA-shape / CWT tuning switches are unknown
+    (ValueError); and nothing is read from the environment: SSQ_NO_H32R=1 leaves a new context on the n_fft 512
+    register kernel."""
+    import torch
+    from ssqueeze_rs_b200._lib import Context
+    from ssqueeze_rs_b200.batch import Engine
+    ctx = Context(0)
+    for name in ("no_h32r", "no_r1024", "no_r256", "no_cwt_fused", "upstream_framing"):
+        ctx.set_option(name, 1)
+        ctx.set_option(name, 0)
+    for name in ("h32r_nw", "istft_nw", "fft128_tc", "cwt_fused_tc", "no_fft128", "no_cwt_prune", "cwt_ws_mb"):
+        with pytest.raises(ValueError):
+            ctx.set_option(name, 1)
+    monkeypatch.setenv("SSQ_NO_H32R", "1")
+    eng = Engine(0)
+    x = torch.randn((2, 5000), device="cuda")
+    eng.ssq_stft(x, np.hanning(512), 512, 32, 30000.0)
+    torch.cuda.synchronize()
+    assert "h32r" in eng.last_kernel_name()
+
+
 
 def test_long_recording_config5_geometry():
     """BASELINE config 5 geometry (10 min @ 30 kHz = 18 M samples per channel, 562 500 frames) on a
