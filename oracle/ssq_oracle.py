@@ -75,11 +75,30 @@ def pad_zeros_stft(x: np.ndarray, n_fft: int) -> np.ndarray:
     return out
 
 
-def _pad_stft(x, n_fft, padtype):
+def pad_upstream_stft(x: np.ndarray, n_fft: int, padtype: str) -> np.ndarray:
+    """Upstream ssqueezepy's framing (old/ssqueezepy/utils/common.py:116-120, padsignal): left n_fft//2 (the larger
+    side for even n_fft), right n_fft-1-n_fft//2, by np.pad.  'reflect' reflects again and again where a pad is longer
+    than the signal (N <= n_fft//2), and a 1-sample signal becomes a constant; 'zero' pads zeros."""
+    left = n_fft // 2
+    return np.pad(x, [left, n_fft - 1 - left], mode="constant" if padtype == "zero" else "reflect")
+
+
+def _pad_stft(x, n_fft, padtype, framing="crate"):
     # stft.rs:25-29 / ssq_stft.rs:124-128: unknown strings fall back to reflect
+    if framing == "upstream":
+        return pad_upstream_stft(x, n_fft, padtype)
+    if framing != "crate":
+        raise ValueError(f"framing must be 'crate' or 'upstream', not {framing!r}")
     if padtype == "zero":
         return pad_zeros_stft(x, n_fft)
     return pad_reflect_stft(x, n_fft)
+
+
+def pad_left(n_fft: int, framing: str = "crate") -> int:
+    """Left pad of a framing: frame f starts at sample f*hop - pad_left, and `istft` unpads there."""
+    if framing not in ("crate", "upstream"):
+        raise ValueError(f"framing must be 'crate' or 'upstream', not {framing!r}")
+    return n_fft // 2 if framing == "upstream" else (n_fft - 1) // 2
 
 
 def _frames(padded: np.ndarray, n_fft: int, hop: int) -> np.ndarray:
@@ -89,11 +108,12 @@ def _frames(padded: np.ndarray, n_fft: int, hop: int) -> np.ndarray:
     return padded[idx]
 
 
-def stft(x, n_fft, hop_length, window, padtype):
+def stft(x, n_fft, hop_length, window, padtype, *, framing="crate"):
     """stft.rs:12-95.  Returns (Sx complex128 [n_fft//2+1, n_frames],
     freqs = linspace(0, 0.5, n_freqs)).  The window is NOT resized: a window
     longer than n_fft is truncated to its first n_fft taps
-    (stft_utils.rs:8), a shorter one makes rustfft panic."""
+    (stft_utils.rs:8), a shorter one makes rustfft panic.  framing="upstream"
+    pads as upstream ssqueezepy does (`pad_upstream_stft`)."""
     x = np.asarray(x, dtype=np.float64)
     window = np.asarray(window, dtype=np.float64)
     if hop_length < 1:
@@ -103,7 +123,7 @@ def stft(x, n_fft, hop_length, window, padtype):
                            "(stft_utils.rs:8, stft.rs:67)")
     if len(x) < 1:
         raise RuntimeError("empty x: usize underflow at stft.rs:33")
-    padded = _pad_stft(x, n_fft, padtype)
+    padded = _pad_stft(x, n_fft, padtype, framing)
     fr = _frames(padded, n_fft, hop_length) * window[:n_fft][None, :]
     n_freqs = n_fft // 2 + 1
     Sx = np.fft.fft(fr, axis=1)[:, :n_freqs].T.copy()
@@ -189,10 +209,11 @@ def reassign_stft(Sx, w, ssq_freqs, squeezing):
 
 def ssq_stft(x, window, n_fft=None, win_len=None, hop_len=1, fs=1.0,
              padtype="reflect", squeezing="sum", gamma=None, *,
-             modulated=False, return_aux=False):
-    """ssq_stft.rs:74-313.  `modulated` / `return_aux` are build-side
+             modulated=False, return_aux=False, framing="crate"):
+    """ssq_stft.rs:74-313.  `modulated` / `return_aux` / `framing` are build-side
     extensions (SURVEY 8a row 10, 8b): modulated multiplies Sx and dSx rows by
-    exp(+2*pi*i*k*(n_fft//2)/n_fft) before squeezing (w is unaffected)."""
+    exp(+2*pi*i*k*(n_fft//2)/n_fft) before squeezing (w is unaffected);
+    framing="upstream" pads as upstream ssqueezepy does (`pad_upstream_stft`)."""
     x = np.asarray(x, dtype=np.float64)
     window = np.asarray(window, dtype=np.float64)
     n = len(x)
@@ -205,7 +226,7 @@ def ssq_stft(x, window, n_fft=None, win_len=None, hop_len=1, fs=1.0,
     if n < 1:
         raise RuntimeError("empty x: usize underflow at ssq_stft.rs:183")
     wsz = fit_window(window, n_fft)
-    padded = _pad_stft(x, n_fft, padtype)
+    padded = _pad_stft(x, n_fft, padtype, framing)
     dwin = diff_window(wsz)
     fr = _frames(padded, n_fft, hop_len)
     n_freqs = n_fft // 2 + 1
@@ -225,13 +246,15 @@ def ssq_stft(x, window, n_fft=None, win_len=None, hop_len=1, fs=1.0,
     return Tx, sf
 
 
-def istft(Sx, window, n_fft=None, win_len=None, hop_len=1, N=None, win_exp=1):
+def istft(Sx, window, n_fft=None, win_len=None, hop_len=1, N=None, win_exp=1, *, framing="crate"):
     """Inverse of `stft` in the Rust framing convention.  Absent from the Rust
     crate (lib.rs:25-32); specified from old/ssqueezepy/_stft.py:184-256 and
     old/ssqueezepy/utils/stft_utils.py:141-191 with modulated=False, and the
-    Rust pad offset (n_fft-1)//2 (stft_utils.rs:22) for unpadding."""
+    Rust pad offset (n_fft-1)//2 (stft_utils.rs:22) for unpadding, or
+    upstream's n_fft//2 with framing="upstream"."""
     Sx = np.asarray(Sx)
     n_fft = n_fft or (Sx.shape[0] - 1) * 2
+    left = pad_left(n_fft, framing)
     n_frames = Sx.shape[1]
     N = N or hop_len * n_frames
     wsz = fit_window(window, n_fft)
@@ -252,7 +275,6 @@ def istft(Sx, window, n_fft=None, win_len=None, hop_len=1, N=None, win_exp=1):
     tiny = np.finfo(np.float64).tiny
     nz = wn > tiny
     xr[nz] /= wn[nz]
-    left = (n_fft - 1) // 2
     return xr[left:left + N]
 
 

@@ -192,15 +192,34 @@ __device__ __forceinline__ float2 csubf(float2 a, float2 b) { return sub2<PK>(a,
 __device__ __forceinline__ float2 cmi(float2 a) { return make_float2(a.y, -a.x); }  // a * (-i)
 __device__ __forceinline__ float2 cpi(float2 a) { return make_float2(-a.y, a.x); }  // a * (+i)
 
+// Internal pad code, never seen at the ABI: reflect padding as upstream ssqueezepy pads, np.pad(mode="reflect"),
+// which reflects again and again where a pad is longer than the signal.  run_stft_family selects it for "reflect"
+// under the upstream_framing option; the crate's own reflect (SSQ_PAD_REFLECT) leaves those samples at zero.  The two
+// differ only for n <= left, where one reflection does not reach every padded sample.
+constexpr int SSQ_PAD_REFLECT_UPSTREAM = 2;
+
 // Padded-signal sample fetch in the reference's STFT framing
-// (stft_utils.rs:19-65): padded index p, left = (n_fft-1)/2.
+// (stft_utils.rs:19-65): padded index p, left = (n_fft-1)/2 (n_fft/2 in upstream framing).
 // `origin`: global index of x[0] (streaming: x holds the samples [origin, ...) of a longer recording of
 // n samples; every index that is read lies inside the carried-over buffer).
+// FOLD = false drops the np.pad fold at compile time: the register kernels' edge-sample function keeps the code it
+// had before the fold existed (run_stft_family does not send them signals of n <= left in upstream reflect).
+template <bool FOLD = true>
 __device__ __forceinline__ float stft_sample(const float* __restrict__ x, int64_t n, int64_t p,
                                              int left, int padtype, int64_t origin = 0) {
   int64_t o = p - left;
   if (o >= 0 && o < n) return __ldg(x + (o - origin));
   if (padtype == SSQ_PAD_ZERO) return 0.f;
+  if (FOLD && padtype == SSQ_PAD_REFLECT_UPSTREAM && (o < 1 - n || o > 2 * n - 2)) {
+    // beyond one reflection (n <= left): np.pad folds the index with period 2 (n - 1), and a 1-sample signal is a
+    // constant.  Then n <= n_fft / 2, so o and n fit in 32 bits, and a stream holds the whole recording (origin 0).
+    const int period = 2 * ((int)n - 1);
+    if (period == 0) return __ldg(x - origin);
+    int r = (int)o % period;
+    if (r < 0) r += period;
+    if (r >= (int)n) r = period - r;
+    return __ldg(x + (r - origin));
+  }
   if (o < 0) {
     int64_t m = -o;  // stft_utils.rs:34-36
     return m < n ? __ldg(x + (m - origin)) : 0.f;

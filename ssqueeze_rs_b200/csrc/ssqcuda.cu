@@ -412,7 +412,9 @@ static ssq_status run_stft_family(ssq_ctx* ctx, const StftCall& c) {
   P.frame0 = c.frame0;
   P.x_origin = c.x_origin;
   P.left = ctx->opt.upstream_framing ? N / 2 : (N - 1) / 2;  // stft_utils.rs:22 | old/ssqueezepy/utils/common.py:116-120
-  P.padtype = c.padtype == SSQ_PAD_ZERO ? SSQ_PAD_ZERO : SSQ_PAD_REFLECT;
+  P.padtype = c.padtype == SSQ_PAD_ZERO ? SSQ_PAD_ZERO
+              : ctx->opt.upstream_framing ? SSQ_PAD_REFLECT_UPSTREAM  // np.pad's reflect (stft_sample)
+              : SSQ_PAD_REFLECT;
   P.win = T.win;
   P.dwin = T.dwin;
   P.wpair = T.wpair;
@@ -440,7 +442,12 @@ static ssq_status run_stft_family(ssq_ctx* ctx, const StftCall& c) {
   bool done = false;
   // diagnostic outputs (aux_*) do not change the kernel selection: the register kernels carry them as a
   // compile-time variant of the same code
+  // a signal of n <= left in upstream reflect needs np.pad's repeated reflection, which only the generic kernel and
+  // the rows path compile in: the register kernels' edge-sample function keeps the crate's one reflection, so that
+  // the code of the benchmarked kernel does not change with it
+  const bool fold = P.padtype == SSQ_PAD_REFLECT_UPSTREAM && P.n <= P.left;
   for (auto launch : {stft_h32r_launch, stft_r1024_launch, stft_r256_launch}) {
+    if (fold) break;
     SSQ_TRY(launch(ctx, P, &done));
     if (done) break;
   }
@@ -974,7 +981,9 @@ __global__ void deinterleave_kernel(const T* __restrict__ in, int64_t n_new, int
 static int64_t stream_frames_ready(const ssq_stream* s, int64_t received) {
   if (received >= s->n_total) return s->n_frames_total;
   const int64_t a = received - s->n_fft + s->left;  // last frame f with f*hop - left + n_fft - 1 < received
-  if (a < 0) return 0;
+  // frame 0 also reads x[left] through the left reflection: in upstream framing with even n_fft that is one sample
+  // past its own last one (left = n_fft - left), so with received == left it is not ready yet
+  if (a < 0 || received <= s->left) return 0;
   return std::min<int64_t>(s->n_frames_total, a / s->hop + 1);
 }
 

@@ -217,7 +217,7 @@ __device__ __forceinline__ void h32r_frame(const StftParams& P, const H32Lane& L
 // instruction cache (the fully inlined version was 88 KB of SASS, 7 % of the issue slots starved).
 __device__ __noinline__ float h32r_edge_sample(const float* x, int64_t n, int64_t p, int left, int padtype,
                                                int64_t origin) {
-  return stft_sample(x, n, p, left, padtype, origin);
+  return stft_sample<false>(x, n, p, left, padtype, origin);
 }
 
 // Warps per CTA, 16 per SM either way.  4 for ssq_stft (16-frame tiles, 128 B row segments, 4 CTAs per SM: half the

@@ -289,11 +289,13 @@ def _flip_tolerant_compare(Tx, To, max_bad_frac=2e-3):
     return float(bad.mean())
 
 
-def check_ssq_device(eng, xd, win, n_fft, hop, fs, channels=None, frame_slices=None, expect_kernel=None, **kw):
+def check_ssq_device(eng, xd, win, n_fft, hop, fs, channels=None, frame_slices=None, expect_kernel=None,
+                     framing="crate", **kw):
     """check_ssq for the batched device API (Engine): the diagnostic twin runs on the whole batch; the oracle runs per
     channel, or -- for recordings too long for it -- on slices of frames (a frame depends on its own n_fft samples
     only, so the oracle is run on the samples of the slice and its interior frames are compared).
-    frame_slices: list of (channel, first_frame, n_frames_in_slice)."""
+    frame_slices: list of (channel, first_frame, n_frames_in_slice).  framing: the oracle's framing ("upstream" for
+    an engine whose context has upstream_framing set)."""
     import torch
     Tx, aux = eng.ssq_stft(xd, win, n_fft, hop, fs, return_aux=True, **kw)
     name = eng.last_kernel_name()
@@ -302,7 +304,7 @@ def check_ssq_device(eng, xd, win, n_fft, hop, fs, channels=None, frame_slices=N
     Tx_plain = eng.ssq_stft(xd, win, n_fft, hop, fs, **kw)
     torch.cuda.synchronize()
     assert torch.equal(Tx, Tx_plain), "diagnostic variant and production kernel disagree: " + name
-    okw = dict(n_fft=n_fft, hop_len=hop, fs=fs, return_aux=True, **kw)
+    okw = dict(n_fft=n_fft, hop_len=hop, fs=fs, return_aux=True, framing=framing, **kw)
     total = dict(bins_total=0, mismatch_total=0, within_edge=0, ill_conditioned=0, below_energy_gate=0, gate_edge=0,
                  unexplained=0, max_err_over_tol=0.0)
 
@@ -325,7 +327,7 @@ def check_ssq_device(eng, xd, win, n_fft, hop, fs, channels=None, frame_slices=N
                 Tx[c].cpu().numpy().astype(np.complex128), To, ao)
     else:
         n = xd.shape[1]
-        left = (n_fft - 1) // 2
+        left = O.pad_left(n_fft, framing)
         for c, f0, nf in frame_slices:
             # global frame f reads samples [f*hop - left, f*hop - left + n_fft).  The slice starts on a frame
             # boundary a = g0*hop, so slice frame j IS global frame g0 + j; frames f0 .. f0+nf-1 lie inside the slice
