@@ -25,6 +25,9 @@
  *    [channels, rows, cols]; they are asynchronous on the context's stream;
  *  - `*_host_f32` entry points take HOST buffers (pinned preferred) and do the
  *    host<->device copies themselves (synchronous at return);
+ *  - streams (`ssq_stream_*` forward, `ssq_istream_*` inverse) take a long
+ *    recording chunk by chunk and are exact at chunk seams; they own their
+ *    buffers, so calls on the same context between two pushes are allowed;
  *  - there is no CPU fallback: without a usable CUDA device every compute
  *    call fails with SSQ_ECUDA.
  */
@@ -331,6 +334,30 @@ ssq_status ssq_feeder_create(ssq_stream* s, int dtype, int depth, ssq_feeder** o
 void ssq_feeder_destroy(ssq_feeder* f);
 ssq_status ssq_feeder_push(ssq_feeder* f, const void* h_chunk, int64_t n_new, float scale, float* d_Tx,
                            int64_t* frames_written);
+
+/* ---- streaming inverse over chunks of frames (DESIGN §3.4c) ------------------ */
+/* The inverse of ssq_stream_*: a stream is created for n_frames_total frames of channels channels; every push hands
+ * over the next n_new (<= max_frames) frames as DEVICE complex64 d_Sx [channels, n_freqs, n_new] -- the layout a
+ * forward push writes, masked or not -- and writes the output samples that became final to d_out,
+ * samples = ssq_istream_samples_after(s, n_new) queried BEFORE the push.  Over all pushes exactly
+ * ssq_istream_total_samples(s) samples are written, equal to the batch call on the whole Sx.
+ * mode 0 = istft (old/ssqueezepy/_stft.py:184-256, ssq_istft_batch_f32's framing and win_exp; n_out <= 0 means
+ * hop * n_frames_total; frames past the batch call's max_hops are accepted and dropped), mode 1 = issq_stft (hop must
+ * be 1; Tx computed with SSQ_FLAG_MODULATED; fs as ssq_issq_stft_batch_f32; one sample per frame).
+ * out_format 0 = fp32 [channels, samples], 1 = fp32 [samples, channels], 2 = int16 [samples, channels] (round to
+ * nearest even, saturated).  Samples are multiplied by (float)(1.0 / scale): scale = 0.195 returns the int16 counts
+ * that a forward stream pushed with scale = 0.195 turned into uV.  The stream owns its buffers: a batch call on the
+ * same context between two pushes does not change what it computes.  Argument errors return SSQ_EINVAL and leave the
+ * stream as it was; ssq_istream_create checks its arguments before it looks at ctx. */
+typedef struct ssq_istream ssq_istream;
+ssq_status ssq_istream_create(ssq_ctx* ctx, int64_t channels, int64_t n_frames_total, int64_t n_out,
+                              int64_t max_frames, const double* window, int64_t win_n, int n_fft, int hop,
+                              int win_exp, int mode, double fs, int out_format, ssq_istream** out);
+void ssq_istream_destroy(ssq_istream* s);
+int64_t ssq_istream_total_samples(const ssq_istream* s);
+int64_t ssq_istream_samples_after(const ssq_istream* s, int64_t n_new);
+ssq_status ssq_istream_push(ssq_istream* s, const float* d_Sx, int64_t n_new, float scale, void* d_out,
+                            int64_t* samples_written);
 
 /* pinned host memory helpers for the host-buffer path */
 ssq_status ssq_host_alloc(void** p, size_t bytes);

@@ -16,6 +16,10 @@ pub struct SsqStream {
 pub struct SsqFeeder {
     _private: [u8; 0],
 }
+#[repr(C)]
+pub struct SsqIstream {
+    _private: [u8; 0],
+}
 
 pub const SSQ_FLAG_MODULATED: c_uint = 1 << 0;
 pub const SSQ_FLAG_NO_FLIPUD: c_uint = 1 << 1;
@@ -77,6 +81,11 @@ extern "C" {
     pub fn ssq_feeder_create(s: *mut SsqStream, dtype: c_int, depth: c_int, out: *mut *mut SsqFeeder) -> c_int;
     pub fn ssq_feeder_destroy(f: *mut SsqFeeder);
     pub fn ssq_feeder_push(f: *mut SsqFeeder, h_chunk: *const c_void, n_new: i64, scale: c_float, d_tx: *mut c_float, frames_written: *mut i64) -> c_int;
+    pub fn ssq_istream_create(ctx: *mut SsqCtx, channels: i64, n_frames_total: i64, n_out: i64, max_frames: i64, window: *const c_double, win_n: i64, n_fft: c_int, hop: c_int, win_exp: c_int, mode: c_int, fs: c_double, out_format: c_int, out: *mut *mut SsqIstream) -> c_int;
+    pub fn ssq_istream_destroy(s: *mut SsqIstream);
+    pub fn ssq_istream_total_samples(s: *const SsqIstream) -> i64;
+    pub fn ssq_istream_samples_after(s: *const SsqIstream, n_new: i64) -> i64;
+    pub fn ssq_istream_push(s: *mut SsqIstream, d_sx: *const c_float, n_new: i64, scale: c_float, d_out: *mut c_void, samples_written: *mut i64) -> c_int;
     pub fn ssq_host_alloc(p: *mut *mut c_void, bytes: usize) -> c_int;
     pub fn ssq_host_free(p: *mut c_void);
     pub fn ssq_memcpy_async(dst: *mut c_void, src: *const c_void, bytes: usize, kind: c_int, cuda_stream: *mut c_void) -> c_int;

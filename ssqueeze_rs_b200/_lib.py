@@ -100,6 +100,12 @@ SIGNATURES = {
     "ssq_feeder_create": (c_int, [c_vp, c_int, c_int, C.POINTER(c_vp)]),
     "ssq_feeder_destroy": (None, [c_vp]),
     "ssq_feeder_push": (c_int, [c_vp, c_vp, c_i64, C.c_float, c_vp, C.POINTER(c_i64)]),
+    "ssq_istream_create": (c_int, [c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_i64, c_int, c_int, c_int, c_int, c_dbl,
+                                   c_int, C.POINTER(c_vp)]),
+    "ssq_istream_destroy": (None, [c_vp]),
+    "ssq_istream_total_samples": (c_i64, [c_vp]),
+    "ssq_istream_samples_after": (c_i64, [c_vp, c_i64]),
+    "ssq_istream_push": (c_int, [c_vp, c_vp, c_i64, C.c_float, c_vp, C.POINTER(c_i64)]),
     "ssq_host_alloc": (c_int, [C.POINTER(c_vp), C.c_size_t]),
     "ssq_host_free": (None, [c_vp]),
     "ssq_memcpy_async": (c_int, [c_vp, c_vp, C.c_size_t, c_int, c_vp]),

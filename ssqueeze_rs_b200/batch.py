@@ -262,7 +262,9 @@ class SsqStftStream:
     float32 CUDA tensors): the B200 replacement of the dask `map_overlap` caller
     (tests/stft_ssq_test.py:218-283 of the reference).  `push(chunk)` returns the frames that
     became complete, complex64 [channels, n_freqs, frames]; concatenated along frames they equal
-    `Engine.ssq_stft` on the whole recording (no re-padding at chunk seams)."""
+    `Engine.ssq_stft` on the whole recording (no re-padding at chunk seams).  Each output can be handed,
+    masked or not, straight to `IstftStream.push` (transform="stft" for istft; modulated=True, hop 1 for
+    issq_stft)."""
 
     def __init__(self, engine: "Engine", channels, n_total, max_chunk, window, n_fft=512, hop_len=32, fs=1.0,
                  padtype="reflect", squeezing="sum", gamma=None, transform="ssq_stft", modulated=False):
@@ -304,6 +306,79 @@ class SsqStftStream:
         if self._h:
             load().ssq_stream_destroy(self._h)
             self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class IstftStream:
+    """Streaming inverse over chunks of frames (ssq_istream_*, DESIGN §3.4c): `push(Sx_chunk)` takes the next frames,
+    complex64 CUDA [channels, n_freqs, frames] as `SsqStftStream` / `RecordingFeeder` yield them, and returns the
+    output samples that became final.  Concatenated over pushes they are `Engine.istft(Sx, window, n_fft, hop_len, N,
+    win_exp)` (transform="istft") or `Engine.issq_stft(Tx, window, n_fft, fs)` (transform="issq_stft", hop_len 1) of
+    the whole Sx / Tx, without ever holding it:
+
+        inv = IstftStream(eng, 384, n_frames, (chunk + 512) // 32 + 2, win, 512, 32, N=n,  # frames of one feeder chunk
+                          out="i16_interleaved", scale=0.195)
+        for Sx in RecordingFeeder(eng, rec, win, 512, 32, chunk=chunk, scale=0.195, transform="stft"):
+            y = inv.push(mask * Sx)      # int16 [samples, 384], the counts of the filtered recording
+
+    out: "f32" -> float32 [channels, samples], "f32_interleaved" -> float32 [samples, channels], "i16_interleaved" ->
+    int16 [samples, channels] (round to nearest even, saturated).  Samples are multiplied by float32(1 / scale)."""
+
+    _FORMATS = {"f32": 0, "f32_interleaved": 1, "i16_interleaved": 2}
+    _TRANSFORMS = {"istft": 0, "issq_stft": 1}
+
+    def __init__(self, engine: "Engine", channels, n_frames_total, max_frames, window, n_fft=512, hop_len=32, N=None,
+                 win_exp=1, transform="istft", fs=1.0, out="f32", scale=1.0):
+        if transform not in self._TRANSFORMS:
+            raise ValueError("transform must be 'istft' or 'issq_stft'")
+        if out not in self._FORMATS:
+            raise ValueError("out must be 'f32', 'f32_interleaved' or 'i16_interleaved'")
+        self.eng, self.out, self.scale = engine, out, float(scale)
+        self.channels, self.n_freqs = int(channels), int(n_fft) // 2 + 1
+        w, wp = _wptr(window)
+        h = C.c_void_p()
+        st = load().ssq_istream_create(engine.ctx.handle, int(channels), int(n_frames_total), int(N or 0),
+                                       int(max_frames), wp, len(w), int(n_fft), int(hop_len), int(win_exp),
+                                       self._TRANSFORMS[transform], float(fs), self._FORMATS[out], C.byref(h))
+        raise_status(st, engine.ctx.handle)
+        self._h = h
+
+    @property
+    def total_samples(self) -> int:
+        return int(load().ssq_istream_total_samples(self._h))
+
+    def push(self, Sx_chunk):
+        import torch
+        assert Sx_chunk.is_cuda and Sx_chunk.dtype == torch.complex64 and Sx_chunk.dim() == 3
+        assert Sx_chunk.shape[:2] == (self.channels, self.n_freqs) and Sx_chunk.is_contiguous()
+        n_new = Sx_chunk.shape[2]
+        k = max(int(load().ssq_istream_samples_after(self._h, n_new)), 0)
+        shape = (self.channels, k) if self.out == "f32" else (k, self.channels)
+        dtype = torch.int16 if self.out == "i16_interleaved" else torch.float32
+        y = torch.empty(shape, dtype=dtype, device=Sx_chunk.device)
+        self.eng._bind_stream()
+        sw = C.c_int64()
+        st = load().ssq_istream_push(self._h, C.c_void_p(Sx_chunk.data_ptr()), n_new, self.scale,
+                                     C.c_void_p(y.data_ptr() if k > 0 else 0), C.byref(sw))
+        raise_status(st, self.eng.ctx.handle)
+        assert sw.value == k
+        return y
+
+    def close(self):
+        if getattr(self, "_h", None):
+            load().ssq_istream_destroy(self._h)
+            self._h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
 
     def __del__(self):
         try:
@@ -374,6 +449,12 @@ class RecordingFeeder:
         with RecordingFeeder(eng, rec, np.hanning(512), scale=0.195, fs=30000.0) as feed:
             for Tx in feed:              # [384, 257, frames of this chunk]
                 ...
+
+    With transform="stft" the chunks are frames of Sx, and `IstftStream` turns them back into samples chunk by chunk
+    (filter in the time-frequency plane, then write the result out):
+
+        for Sx in RecordingFeeder(eng, rec, win, 512, 32, chunk=1 << 18, scale=0.195, transform="stft"):
+            y = inv.push(mask * Sx)      # inv = IstftStream(..., out="i16_interleaved", scale=0.195)
     """
 
     def __init__(self, engine: "Engine", recording, window, n_fft=512, hop_len=32, fs=1.0, chunk=1 << 16, scale=1.0,

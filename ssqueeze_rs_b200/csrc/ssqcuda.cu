@@ -11,6 +11,7 @@
 #include "istft_h32.cuh"
 #include "istft_r1024.cuh"
 #include "istft_r256.cuh"
+#include "istream_kernels.cuh"
 #include "cwt_kernels.cuh"
 #include "ridge_kernels.cuh"
 
@@ -29,7 +30,7 @@ static const double kEps64 = 2.2204460492503131e-16;
 // ===========================================================================
 extern "C" const char* ssq_version(void) {
   return "ssqcuda 0.3 (B200 sm_100a; stft, ssq_stft, istft, issq_stft, cwt, cwt_simd, ssq_cwt, icwt, issq_cwt, "
-         "ssq_stft streaming, ridge extraction)";
+         "ssq_stft streaming, istft / issq_stft streaming, ridge extraction)";
 }
 
 // lib.rs:16-19
@@ -547,37 +548,22 @@ static inline int istft_left(const ssq_ctx* ctx, int n_fft) {
   return ctx->opt.upstream_framing ? n_fft / 2 : (n_fft - 1) / 2;
 }
 
-extern "C" ssq_status ssq_istft_batch_f32(ssq_ctx* ctx, const float* d_Sx, int64_t channels, int64_t n_freqs,
-                                          int64_t n_frames, const double* window, int64_t win_n, int n_fft,
-                                          int hop, int64_t n_out, int win_exp, float* d_xout) {
-  if (!ctx) return ssq_fail(nullptr, SSQ_EINVAL, "ctx is NULL");
-  if (!d_Sx || !d_xout || !window || win_n < 1) return ssq_fail(ctx, SSQ_EINVAL, "NULL/empty argument");
-  SSQ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  if (n_fft <= 0) n_fft = (int)(n_freqs - 1) * 2;  // _stft.py:229
-  if (n_fft < 2 || n_fft / 2 + 1 != n_freqs)
-    return ssq_fail(ctx, SSQ_EINVAL, "Sx has %lld rows but n_fft=%d needs %d", (long long)n_freqs, n_fft,
-                    n_fft / 2 + 1);
-  if (hop < 1 || n_frames < 1 || channels < 1 || win_exp < 0)
-    return ssq_fail(ctx, SSQ_EINVAL, "bad hop/n_frames/channels/win_exp");
-  if (n_out <= 0) n_out = (int64_t)hop * n_frames;  // _stft.py:231
-  std::vector<double> wfit = ssqhost::fit_window(window, win_n, n_fft);
-  StftTables T;
-  SSQ_TRY(stft_tables(ctx, wfit, TAB_ISTFT, win_exp, &T));
-  const int64_t L = n_out + n_fft - 1;
-  const int64_t max_hops = (L - n_fft) / hop + 1;
-  SSQ_TRY(devbuf_reserve(ctx, ctx->ws_misc, (size_t)channels * L * sizeof(float)));
-  SSQ_CUDA_TRY(ctx, cudaMemsetAsync(ctx->ws_misc.p, 0, (size_t)channels * L * sizeof(float), ctx->stream));
-
+// Overlap-adds the windowed inverse transforms of frames [0, n_use) of Sx (complex64 [channels, n_freqs, n_frames])
+// into xacc ([channels, L], zeroed by the caller; frame f lands at f * hop, and (n_use - 1) * hop + n_fft <= L): the
+// register tile kernels, then the row passes, then the generic kernel.  The window-norm division is the caller's.
+// ev0 / ev1 bracket the dispatch and last_kernel names the kernel that ran.  Shared by the batch call and the stream.
+static ssq_status istft_ola_run(ssq_ctx* ctx, const float2* Sx, int64_t channels, int64_t n_freqs, int64_t n_frames,
+                                int64_t n_use, int n_fft, int hop, const StftTables& T, float* xacc, int64_t L) {
   Istft32Params Q;
   memset(&Q, 0, sizeof(Q));
-  Q.Sx = (const float2*)d_Sx;
+  Q.Sx = Sx;
   Q.channels = (int)channels;
   Q.n_frames = n_frames;
-  Q.n_use = std::min<int64_t>(n_frames, max_hops);
+  Q.n_use = n_use;
   Q.L = L;
   Q.wa = T.wa;
   Q.tw = T.tw;
-  Q.xacc = (float*)ctx->ws_misc.p;
+  Q.xacc = xacc;
   Q.hop = hop;
   Q.n_fft = n_fft;
   SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
@@ -618,6 +604,31 @@ extern "C" ssq_status ssq_istft_batch_f32(ssq_ctx* ctx, const float* d_Sx, int64
   }
   SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
   ctx->ev_valid = true;
+  return SSQ_OK;
+}
+
+extern "C" ssq_status ssq_istft_batch_f32(ssq_ctx* ctx, const float* d_Sx, int64_t channels, int64_t n_freqs,
+                                          int64_t n_frames, const double* window, int64_t win_n, int n_fft,
+                                          int hop, int64_t n_out, int win_exp, float* d_xout) {
+  if (!ctx) return ssq_fail(nullptr, SSQ_EINVAL, "ctx is NULL");
+  if (!d_Sx || !d_xout || !window || win_n < 1) return ssq_fail(ctx, SSQ_EINVAL, "NULL/empty argument");
+  SSQ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  if (n_fft <= 0) n_fft = (int)(n_freqs - 1) * 2;  // _stft.py:229
+  if (n_fft < 2 || n_fft / 2 + 1 != n_freqs)
+    return ssq_fail(ctx, SSQ_EINVAL, "Sx has %lld rows but n_fft=%d needs %d", (long long)n_freqs, n_fft,
+                    n_fft / 2 + 1);
+  if (hop < 1 || n_frames < 1 || channels < 1 || win_exp < 0)
+    return ssq_fail(ctx, SSQ_EINVAL, "bad hop/n_frames/channels/win_exp");
+  if (n_out <= 0) n_out = (int64_t)hop * n_frames;  // _stft.py:231
+  std::vector<double> wfit = ssqhost::fit_window(window, win_n, n_fft);
+  StftTables T;
+  SSQ_TRY(stft_tables(ctx, wfit, TAB_ISTFT, win_exp, &T));
+  const int64_t L = n_out + n_fft - 1;
+  const int64_t max_hops = (L - n_fft) / hop + 1;
+  SSQ_TRY(devbuf_reserve(ctx, ctx->ws_misc, (size_t)channels * L * sizeof(float)));
+  SSQ_CUDA_TRY(ctx, cudaMemsetAsync(ctx->ws_misc.p, 0, (size_t)channels * L * sizeof(float), ctx->stream));
+  SSQ_TRY(istft_ola_run(ctx, (const float2*)d_Sx, channels, n_freqs, n_frames, std::min<int64_t>(n_frames, max_hops),
+                        n_fft, hop, T, (float*)ctx->ws_misc.p, L));
   dim3 g((unsigned)((n_out + ISTFT_FIN_PER_BLOCK - 1) / ISTFT_FIN_PER_BLOCK), (unsigned)channels);
   istft_finalize_kernel<<<g, 256, 0, ctx->stream>>>((const float*)ctx->ws_misc.p, L, n_out, n_fft, hop,
                                                     istft_left(ctx, n_fft), max_hops, T.wpow, d_xout);
@@ -1262,6 +1273,212 @@ extern "C" ssq_status ssq_feeder_push(ssq_feeder* f, const void* h_chunk, int64_
   f->pushes++;
   if (st == SSQ_OK && er != cudaSuccess) return ssq_fail(ctx, SSQ_ECUDA, "cudaEventRecord: %s", cudaGetErrorString(er));
   return st;
+}
+
+// ===========================================================================
+// Streaming inverse (DESIGN §3.4c): istft / issq_stft over chunks of frames, the inverse of ssq_stream_*.
+// istft: padded position p = f * hop + m of frame f belongs to output p - left.  Once r of the used frames (those
+// below n_use = min(n_frames_total, max_hops), the batch call's clamp) have arrived, every p < r * hop is final; the
+// positions the next frames still reach keep their undivided partial sums in a carry of at most n_fft - hop samples
+// per channel.  issq_stft: output j is frame j, final at once.
+// ===========================================================================
+struct ssq_istream {
+  ssq_ctx* ctx;
+  int64_t channels, n_frames_total, n_out, max_frames;
+  std::vector<double> wfit;
+  int n_fft, hop, win_exp, mode, out_format, left;
+  int64_t max_hops, n_use;
+  float issq_scale;          // mode 1: 2 / (w[n_fft/2] fs), as ssq_issq_stft_batch_f32
+  float inv_scale;           // (float)(1.0 / scale) of the creation
+  int64_t received = 0;      // frames pushed
+  int64_t emitted = 0;       // samples written
+  int64_t clen = 0;          // valid samples of carry[cur]
+  int64_t cstride = 1;       // max(1, n_fft - hop)
+  float* acc = nullptr;      // [channels, (max_frames - 1) * hop + n_fft]: this push's overlap-add
+  float* carry[2] = {nullptr, nullptr};
+  int cur = 0;
+};
+
+// samples final once `frames` frames have been pushed
+static int64_t istream_ready(const ssq_istream* s, int64_t frames) {
+  if (s->mode == 1) return std::min(frames, s->n_out);
+  const int64_t r = std::min(frames, s->n_use);
+  if (r >= s->n_use) return s->n_out;
+  return std::min<int64_t>(s->n_out, std::max<int64_t>(0, r * s->hop - s->left));
+}
+
+extern "C" void ssq_istream_destroy(ssq_istream* s) {
+  if (!s) return;
+  cudaSetDevice(s->ctx->device);
+  cudaStreamSynchronize(s->ctx->stream);
+  if (s->acc) cudaFree(s->acc);
+  for (int i = 0; i < 2; ++i)
+    if (s->carry[i]) cudaFree(s->carry[i]);
+  delete s;
+}
+
+extern "C" ssq_status ssq_istream_create(ssq_ctx* ctx, int64_t channels, int64_t n_frames_total, int64_t n_out,
+                                         int64_t max_frames, const double* window, int64_t win_n, int n_fft, int hop,
+                                         int win_exp, int mode, double fs, int out_format, ssq_istream** out) {
+  // argument checks first, all on the host: they need neither a context nor a device
+  if (!out) return ssq_fail(ctx, SSQ_EINVAL, "ssq_istream_create: out is NULL");
+  *out = nullptr;
+  if (mode != 0 && mode != 1)
+    return ssq_fail(ctx, SSQ_EINVAL, "istream mode %d: must be 0 (istft) or 1 (issq_stft)", mode);
+  if (out_format < ISTREAM_F32 || out_format > ISTREAM_I16_INTERLEAVED)
+    return ssq_fail(ctx, SSQ_EINVAL,
+                    "istream out_format %d: must be 0 (fp32 [channels, samples]), 1 (fp32 [samples, channels]) or "
+                    "2 (int16 [samples, channels])",
+                    out_format);
+  if (!window || win_n < 1) return ssq_fail(ctx, SSQ_EINVAL, "istream: NULL/empty window");
+  if (channels < 1 || channels > 65535 || n_frames_total < 1 || max_frames < 1 || n_fft < 2 || hop < 1 ||
+      win_exp < 0)
+    return ssq_fail(ctx, SSQ_EINVAL,
+                    "istream: bad sizes (channels=%lld in [1, 65535], n_frames_total=%lld, max_frames=%lld, n_fft=%d, "
+                    "hop=%d, win_exp=%d)",
+                    (long long)channels, (long long)n_frames_total, (long long)max_frames, n_fft, hop, win_exp);
+  if (mode == 1 && hop != 1)
+    return ssq_fail(ctx, SSQ_EINVAL, "istream issq_stft: inversion with `hop_len != 1` is unsupported (hop=%d)", hop);
+  if (mode == 1 && n_out > 0 && n_out != n_frames_total)
+    return ssq_fail(ctx, SSQ_EINVAL, "istream issq_stft: n_out=%lld, but issq_stft returns one sample per frame (%lld)",
+                    (long long)n_out, (long long)n_frames_total);
+  if (mode == 1 && !(fs > 0.0)) return ssq_fail(ctx, SSQ_EINVAL, "istream issq_stft: fs must be > 0");
+  if (!ctx) return ssq_fail(nullptr, SSQ_EINVAL, "ctx is NULL");
+  SSQ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  ssq_istream* s = new (std::nothrow) ssq_istream();
+  if (!s) return ssq_fail(ctx, SSQ_ENOMEM, "out of host memory");
+  s->ctx = ctx;
+  s->channels = channels;
+  s->n_frames_total = n_frames_total;
+  s->n_out = n_out > 0 ? n_out : (int64_t)hop * n_frames_total;  // _stft.py:231
+  s->max_frames = max_frames;
+  s->wfit = ssqhost::fit_window(window, win_n, n_fft);
+  s->n_fft = n_fft;
+  s->hop = hop;
+  s->win_exp = win_exp;
+  s->mode = mode;
+  s->out_format = out_format;
+  s->left = istft_left(ctx, n_fft);
+  s->max_hops = (s->n_out - 1) / hop + 1;  // (L - n_fft) / hop + 1 with L = n_out + n_fft - 1
+  s->n_use = std::min(n_frames_total, s->max_hops);
+  s->issq_scale = (float)(2.0 / (s->wfit[(size_t)(n_fft / 2)] * fs));
+  s->inv_scale = 1.f;
+  s->cstride = std::max(1, n_fft - hop);
+  if (mode == 0) {
+    const int64_t la = (std::min(max_frames, s->n_use) - 1) * hop + n_fft;
+    cudaError_t e = cudaMalloc((void**)&s->acc, (size_t)channels * la * sizeof(float));
+    for (int i = 0; i < 2 && e == cudaSuccess; ++i)
+      e = cudaMalloc((void**)&s->carry[i], (size_t)channels * s->cstride * sizeof(float));
+    if (e != cudaSuccess) {
+      (void)cudaGetLastError();
+      ssq_istream_destroy(s);
+      return ssq_fail(ctx, SSQ_ENOMEM, "istream buffers (%lld x %lld floats): %s", (long long)channels, (long long)la,
+                      cudaGetErrorString(e));
+    }
+  }
+  *out = s;
+  return SSQ_OK;
+}
+
+extern "C" int64_t ssq_istream_total_samples(const ssq_istream* s) { return s ? s->n_out : 0; }
+
+extern "C" int64_t ssq_istream_samples_after(const ssq_istream* s, int64_t n_new) {
+  if (!s || n_new < 0) return 0;
+  return istream_ready(s, std::min(s->n_frames_total, s->received + n_new)) - s->emitted;
+}
+
+extern "C" ssq_status ssq_istream_push(ssq_istream* s, const float* d_Sx, int64_t n_new, float scale, void* d_out,
+                                       int64_t* samples_written) {
+  if (!s) return ssq_fail(nullptr, SSQ_EINVAL, "istream is NULL");
+  ssq_ctx* ctx = s->ctx;
+  if (samples_written) *samples_written = 0;
+  // every check before the first change of state: a refused push leaves the stream as it was
+  if (n_new < 0 || n_new > s->max_frames)
+    return ssq_fail(ctx, SSQ_EINVAL, "push of %lld frames (max_frames %lld)", (long long)n_new, (long long)s->max_frames);
+  if (s->received + n_new > s->n_frames_total)
+    return ssq_fail(ctx, SSQ_EINVAL, "push of %lld frames after %lld: more frames than n_frames_total (%lld)",
+                    (long long)n_new, (long long)s->received, (long long)s->n_frames_total);
+  if (n_new > 0 && !d_Sx) return ssq_fail(ctx, SSQ_EINVAL, "d_Sx is NULL");
+  if (!(scale != 0.f) || !std::isfinite(scale)) return ssq_fail(ctx, SSQ_EINVAL, "scale must be finite and non-zero");
+  const int64_t n_emit = istream_ready(s, s->received + n_new) - s->emitted;
+  if (n_emit > 0 && !d_out)
+    return ssq_fail(ctx, SSQ_EINVAL, "d_out is NULL but %lld samples are ready", (long long)n_emit);
+  SSQ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  const float inv_scale = (float)(1.0 / (double)scale);
+  const int64_t n_freqs = s->n_fft / 2 + 1;
+  const dim3 blk(32, 8);
+  const unsigned gy = (unsigned)((s->channels + 31) / 32);
+  if (s->mode == 1) {
+    if (n_new > 0) {
+      dim3 g((unsigned)((n_new + 31) / 32), gy);
+      SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+      const float2* Tx = (const float2*)d_Sx;
+      if (s->out_format == ISTREAM_F32)
+        istream_issq_kernel<ISTREAM_F32><<<g, blk, 0, ctx->stream>>>(Tx, s->channels, n_freqs, n_new, s->issq_scale,
+                                                                      inv_scale, d_out);
+      else if (s->out_format == ISTREAM_F32_INTERLEAVED)
+        istream_issq_kernel<ISTREAM_F32_INTERLEAVED><<<g, blk, 0, ctx->stream>>>(Tx, s->channels, n_freqs, n_new,
+                                                                                  s->issq_scale, inv_scale, d_out);
+      else
+        istream_issq_kernel<ISTREAM_I16_INTERLEAVED><<<g, blk, 0, ctx->stream>>>(Tx, s->channels, n_freqs, n_new,
+                                                                                  s->issq_scale, inv_scale, d_out);
+      SSQ_TRY(ssq_check_launch(ctx, "istream_issq_kernel"));
+      ctx->last_kernel = "istream_issq_kernel";
+      SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+      ctx->ev_valid = true;
+    }
+    s->received += n_new;
+    s->emitted += n_emit;
+    if (samples_written) *samples_written = n_emit;
+    return SSQ_OK;
+  }
+  // frames of this push that the batch call would use; the rest (beyond max_hops) are dropped as it drops them
+  const int64_t u = std::max<int64_t>(0, std::min(n_new, s->n_use - s->received));
+  if (u > 0) {
+    StftTables T;  // re-checked every push: a batch call in between may have replaced the context's tables
+    SSQ_TRY(stft_tables(ctx, s->wfit, TAB_ISTFT, s->win_exp, &T));
+    const int64_t La = (u - 1) * s->hop + s->n_fft;
+    SSQ_CUDA_TRY(ctx, cudaMemsetAsync(s->acc, 0, (size_t)s->channels * La * sizeof(float), ctx->stream));
+    SSQ_TRY(istft_ola_run(ctx, (const float2*)d_Sx, s->channels, n_freqs, n_new, u, s->n_fft, s->hop, T, s->acc, La));
+    IstreamFinParams P;
+    memset(&P, 0, sizeof(P));
+    P.A = s->acc;
+    P.La = La;
+    P.Cin = s->carry[s->cur];
+    P.Cout = s->carry[s->cur ^ 1];
+    P.cstride = s->cstride;
+    P.clen_in = s->clen;
+    P.clen_out = s->received + u < s->n_use ? std::max(0, s->n_fft - s->hop) : 0;
+    P.q_carry = u * s->hop;
+    P.channels = s->channels;
+    P.n_emit = n_emit;
+    P.base = s->received * s->hop;
+    P.q0 = s->emitted + s->left - P.base;  // >= 0: earlier pushes emitted exactly the positions below base
+    P.n_fft = s->n_fft;
+    P.hop = s->hop;
+    P.max_hops = s->max_hops;
+    P.wpow = T.wpow;
+    P.inv_scale = inv_scale;
+    P.out = d_out;
+    P.nb_out = (int)((n_emit + ISTREAM_TILE - 1) / ISTREAM_TILE);
+    const int64_t nb = P.nb_out + (P.clen_out + ISTREAM_TILE - 1) / ISTREAM_TILE;
+    if (nb > 0) {
+      dim3 g((unsigned)nb, gy);
+      if (s->out_format == ISTREAM_F32)
+        istream_finalize_kernel<ISTREAM_F32><<<g, blk, 0, ctx->stream>>>(P);
+      else if (s->out_format == ISTREAM_F32_INTERLEAVED)
+        istream_finalize_kernel<ISTREAM_F32_INTERLEAVED><<<g, blk, 0, ctx->stream>>>(P);
+      else
+        istream_finalize_kernel<ISTREAM_I16_INTERLEAVED><<<g, blk, 0, ctx->stream>>>(P);
+      SSQ_TRY(ssq_check_launch(ctx, "istream_finalize_kernel"));
+    }
+    s->cur ^= 1;
+    s->clen = P.clen_out;
+  }
+  s->received += n_new;
+  s->emitted += n_emit;
+  if (samples_written) *samples_written = n_emit;
+  return SSQ_OK;
 }
 
 #include "cwt_host.inl"

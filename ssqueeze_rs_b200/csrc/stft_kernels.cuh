@@ -387,18 +387,38 @@ __global__ void __launch_bounds__(256) istft_ola_kernel(const IstftParams P) {
 #define ISTFT_FIN_MAX_HOP 1024
 // The window norm wn(p) = sum_j w^(a+1)[p - j hop] only depends on p mod hop once every frame
 // that covers p exists (p >= n_fft-1 and p/hop < max_hops): one table of `hop` sums per block
-// serves those samples, the two ends of the signal take the explicit loop.
+// serves those samples, the two ends of the signal take the explicit loop.  The batch finalize and
+// the streaming one (istream_kernels.cuh) both go through these two functions, so that they divide
+// every sample by the same float.
+// (callers build the table only when hop <= ISTFT_FIN_MAX_HOP, then synchronise)
+__device__ __forceinline__ void istft_wn_table(float* tab, int n_fft, int hop, const float* __restrict__ wpow, int tid,
+                                               int nthreads) {
+  for (int r = tid; r < hop; r += nthreads) {
+    float s = 0.f;
+    for (int m = r; m < n_fft; m += hop) s += wpow[m];
+    tab[r] = s;
+  }
+}
+
+__device__ __forceinline__ float istft_window_norm(int64_t p, int n_fft, int hop, int64_t max_hops, const float* tab,
+                                                   const float* __restrict__ wpow) {
+  int64_t jhi = p / hop;
+  if (hop <= ISTFT_FIN_MAX_HOP && p >= n_fft - 1 && jhi <= max_hops - 1) return tab[(int)(p - jhi * hop)];
+  if (jhi > max_hops - 1) jhi = max_hops - 1;
+  const int64_t jlo = (p - n_fft + 1 <= 0) ? 0 : (p - n_fft + hop) / hop;
+  float wn = 0.f;
+  for (int64_t j = jlo; j <= jhi; ++j) wn += wpow[p - j * hop];
+  return wn;
+}
+
+#define ISTFT_WN_TINY 1.17549435e-38f  // np.finfo(float32).tiny guard (_stft.py:246-251)
+
 __global__ void __launch_bounds__(256) istft_finalize_kernel(const float* __restrict__ xacc, int64_t L, int64_t n_out,
                                                              int n_fft, int hop, int left, int64_t max_hops,
                                                              const float* __restrict__ wpow, float* __restrict__ out) {
   __shared__ float tab[ISTFT_FIN_MAX_HOP];
-  const bool use_tab = hop <= ISTFT_FIN_MAX_HOP;
-  if (use_tab) {
-    for (int r = threadIdx.x; r < hop; r += blockDim.x) {
-      float s = 0.f;
-      for (int m = r; m < n_fft; m += hop) s += wpow[m];
-      tab[r] = s;
-    }
+  if (hop <= ISTFT_FIN_MAX_HOP) {
+    istft_wn_table(tab, n_fft, hop, wpow, threadIdx.x, blockDim.x);
     __syncthreads();
   }
   const int64_t c = blockIdx.y;
@@ -407,18 +427,9 @@ __global__ void __launch_bounds__(256) istft_finalize_kernel(const float* __rest
     const int64_t n = n0 + i;
     if (n >= n_out) break;
     const int64_t p = n + left;
-    int64_t jhi = p / hop;
-    float wn;
-    if (use_tab && p >= n_fft - 1 && jhi <= max_hops - 1) {
-      wn = tab[(int)(p - jhi * hop)];
-    } else {
-      if (jhi > max_hops - 1) jhi = max_hops - 1;
-      const int64_t jlo = (p - n_fft + 1 <= 0) ? 0 : (p - n_fft + hop) / hop;
-      wn = 0.f;
-      for (int64_t j = jlo; j <= jhi; ++j) wn += wpow[p - j * hop];
-    }
+    const float wn = istft_window_norm(p, n_fft, hop, max_hops, tab, wpow);
     float v = xacc[(size_t)c * L + p];
-    if (wn > 1.17549435e-38f) v /= wn;  // np.finfo(float32).tiny guard (_stft.py:246-251)
+    if (wn > ISTFT_WN_TINY) v /= wn;
     out[(size_t)c * n_out + n] = v;
   }
 }
