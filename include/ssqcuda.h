@@ -190,10 +190,18 @@ ssq_status ssq_issq_cwt_f64(ssq_ctx* ctx, const double* Tx, int64_t ns, int64_t 
                             const double* scales, double* x);
 
 /* `issq_cwt` with curve bands (old/ssqueezepy/_ssq_cwt.py:313-402): component c of column j sums Re Tx over the rows
- * cc[j][c] - cw[j][c] .. cc[j][c] + cw[j][c] (clipped; cc == -1: no curve at that column); the last output row is
- * the residual (rows no band covers).  cc, cw: int32 [n][K], 1 <= K <= 16.  x: float64 [K + 1][n]. */
+ * lower .. upper (inclusive), upper = clip(cc[j][c] + cw[j][c], 0, ns), lower = clip(cc[j][c] - cw[j][c], 0, ns)
+ * (in 64 bits; cc == -1: no curve at that column); each component is summed from the original Tx, so bands may
+ * overlap; the last output row is the residual (rows no band covers).  cc, cw: int32 [n][K], 1 <= K <= 16
+ * (SSQ_EUNSUPPORTED otherwise).  x: float64 [K + 1][n]. */
 ssq_status ssq_issq_cwt_components_f64(ssq_ctx* ctx, const double* Tx, int64_t ns, int64_t n, int wavelet,
                                        const double* scales, const int* cc, const int* cw, int K, double* x);
+/* `issq_stft` with curve bands (upstream's issq_stft(Tx, ..., cc, cw), old/ssqueezepy/_ssq_stft.py:139-198): the
+ * bands of ssq_issq_cwt_components_f64 over the n_freqs rows, times 2 / (window_fit[n_fft/2] * fs); hop must be 1.
+ * Tx complex128 [n_freqs, n_frames]; cc, cw int32 [n_frames][K]; y float64 [K + 1][n_frames], row K the residual. */
+ssq_status ssq_issq_stft_components_f64(ssq_ctx* ctx, const double* Tx, int64_t n_freqs, int64_t n_frames,
+                                        const double* window, int64_t win_n, int n_fft, int hop, double fs,
+                                        const int32_t* cc, const int32_t* cw, int K, double* y);
 
 /* ---- batched throughput path (device buffers, fp32 / complex64) ---------- */
 /* replaces the per-channel Python loop around `_rs.ssq_stft`
@@ -226,6 +234,13 @@ ssq_status ssq_istft_batch_f32(ssq_ctx* ctx, const float* d_Sx, int64_t channels
 ssq_status ssq_issq_stft_batch_f32(ssq_ctx* ctx, const float* d_Tx, int64_t channels,
                                    int64_t n_freqs, int64_t n_frames, const double* window,
                                    int64_t win_n, int n_fft, double fs, float* d_y);
+/* same bands as ssq_issq_cwt_components_batch_f32 on an issq_stft map (hop 1, modulated Tx), times the factor of
+ * ssq_issq_stft_batch_f32: d_Tx complex64 [channels, n_freqs, n_frames]; d_cc, d_cw DEVICE int32
+ * [channels, n_frames, K]; d_y fp32 [channels, K + 1, n_frames], row K the residual */
+ssq_status ssq_issq_stft_components_batch_f32(ssq_ctx* ctx, const float* d_Tx, int64_t channels,
+                                              int64_t n_freqs, int64_t n_frames, const double* window,
+                                              int64_t win_n, int n_fft, double fs, const int32_t* d_cc,
+                                              const int32_t* d_cw, int K, float* d_y);
 /* d_Wx / d_dWx complex64 [channels, ns, n] (d_dWx may be NULL) */
 ssq_status ssq_cwt_batch_f32(ssq_ctx* ctx, const float* d_x, int64_t channels, int64_t n,
                              int64_t x_stride, int wavelet, const double* scales, int64_t ns,
@@ -252,6 +267,13 @@ ssq_status ssq_icwt_batch_f32(ssq_ctx* ctx, const float* d_Wx, int64_t channels,
 /* d_Tx complex64 [channels, ns, n] -> d_x fp32 [channels, n] */
 ssq_status ssq_issq_cwt_batch_f32(ssq_ctx* ctx, const float* d_Tx, int64_t channels, int64_t ns, int64_t n,
                                   int wavelet, const double* scales, float* d_x);
+/* curve bands on the device (the rule of ssq_issq_cwt_components_f64, clipped by the kernel): d_Tx complex64
+ * [channels, ns, n]; d_cc, d_cw DEVICE int32 [channels, n, K] (the layout of ssq_extract_ridges_batch's
+ * d_ridge_idxs), 1 <= K <= 16; d_x fp32 [channels, K + 1, n], row K the residual.  Channel c equals the one-channel
+ * call bit for bit, and one band covering every row equals ssq_issq_cwt_batch_f32 bit for bit. */
+ssq_status ssq_issq_cwt_components_batch_f32(ssq_ctx* ctx, const float* d_Tx, int64_t channels, int64_t ns,
+                                             int64_t n, int wavelet, const double* scales, const int32_t* d_cc,
+                                             const int32_t* d_cw, int K, float* d_x);
 
 /* ---- wavelet generators (SURVEY 8f rank 2) --------------------------------------------------------------
  * The functions src/ssqueeze/_rs.pyi:91-132 declares: `morlet`, `morlet_freq`, `morlet_time` (rust/src/wavelets/

@@ -54,16 +54,19 @@ extern "C" {
     pub fn ssq_cwt_admissibility(wavelet: c_int, css: *mut c_double) -> c_int;
     pub fn ssq_issq_cwt_f64(ctx: *mut SsqCtx, tx: *const c_double, ns: i64, n: i64, wavelet: c_int, scales: *const c_double, x: *mut c_double) -> c_int;
     pub fn ssq_issq_cwt_components_f64(ctx: *mut SsqCtx, tx: *const c_double, ns: i64, n: i64, wavelet: c_int, scales: *const c_double, cc: *const c_int, cw: *const c_int, k: c_int, x: *mut c_double) -> c_int;
+    pub fn ssq_issq_stft_components_f64(ctx: *mut SsqCtx, tx: *const c_double, n_freqs: i64, n_frames: i64, window: *const c_double, win_n: i64, n_fft: c_int, hop: c_int, fs: c_double, cc: *const i32, cw: *const i32, k: c_int, y: *mut c_double) -> c_int;
     pub fn ssq_ssq_stft_batch_f32(ctx: *mut SsqCtx, d_x: *const c_float, channels: i64, n: i64, x_stride: i64, window: *const c_double, win_n: i64, n_fft: c_int, hop: c_int, fs: c_double, padtype: c_int, squeezing: c_int, gamma: c_double, flags: c_uint, d_tx: *mut c_float) -> c_int;
     pub fn ssq_ssq_stft_batch_diag_f32(ctx: *mut SsqCtx, d_x: *const c_float, channels: i64, n: i64, x_stride: i64, window: *const c_double, win_n: i64, n_fft: c_int, hop: c_int, fs: c_double, padtype: c_int, squeezing: c_int, gamma: c_double, flags: c_uint, d_tx: *mut c_float, d_sx: *mut c_float, d_dsx: *mut c_float, d_w: *mut c_float, d_kb: *mut i32) -> c_int;
     pub fn ssq_stft_batch_f32(ctx: *mut SsqCtx, d_x: *const c_float, channels: i64, n: i64, x_stride: i64, window: *const c_double, win_n: i64, n_fft: c_int, hop: c_int, padtype: c_int, d_sx: *mut c_float) -> c_int;
     pub fn ssq_istft_batch_f32(ctx: *mut SsqCtx, d_sx: *const c_float, channels: i64, n_freqs: i64, n_frames: i64, window: *const c_double, win_n: i64, n_fft: c_int, hop: c_int, n_out: i64, win_exp: c_int, d_xout: *mut c_float) -> c_int;
     pub fn ssq_issq_stft_batch_f32(ctx: *mut SsqCtx, d_tx: *const c_float, channels: i64, n_freqs: i64, n_frames: i64, window: *const c_double, win_n: i64, n_fft: c_int, fs: c_double, d_y: *mut c_float) -> c_int;
+    pub fn ssq_issq_stft_components_batch_f32(ctx: *mut SsqCtx, d_tx: *const c_float, channels: i64, n_freqs: i64, n_frames: i64, window: *const c_double, win_n: i64, n_fft: c_int, fs: c_double, d_cc: *const i32, d_cw: *const i32, k: c_int, d_y: *mut c_float) -> c_int;
     pub fn ssq_cwt_batch_f32(ctx: *mut SsqCtx, d_x: *const c_float, channels: i64, n: i64, x_stride: i64, wavelet: c_int, scales: *const c_double, ns: i64, dt: c_double, padtype: c_int, flags: c_uint, d_wx: *mut c_float, d_dwx: *mut c_float) -> c_int;
     pub fn ssq_ssq_cwt_batch_f32(ctx: *mut SsqCtx, d_x: *const c_float, channels: i64, n: i64, x_stride: i64, wavelet: c_int, scales: *const c_double, ns: i64, dt: c_double, freq_dist: c_int, padtype: c_int, squeezing: c_int, maprange: c_int, gamma: c_double, flags: c_uint, d_tx: *mut c_float, ssq_freqs: *mut c_double) -> c_int;
     pub fn ssq_ssq_cwt_batch_diag_f32(ctx: *mut SsqCtx, d_x: *const c_float, channels: i64, n: i64, x_stride: i64, wavelet: c_int, scales: *const c_double, ns: i64, dt: c_double, freq_dist: c_int, padtype: c_int, squeezing: c_int, maprange: c_int, gamma: c_double, flags: c_uint, d_tx: *mut c_float, ssq_freqs: *mut c_double, d_w: *mut c_float, d_kb: *mut i32) -> c_int;
     pub fn ssq_icwt_batch_f32(ctx: *mut SsqCtx, d_wx: *const c_float, channels: i64, ns: i64, n_cols: i64, wavelet: c_int, scales: *const c_double, one_int: c_int, x_len: i64, x_mean: c_double, flags: c_uint, d_x: *mut c_float) -> c_int;
     pub fn ssq_issq_cwt_batch_f32(ctx: *mut SsqCtx, d_tx: *const c_float, channels: i64, ns: i64, n: i64, wavelet: c_int, scales: *const c_double, d_x: *mut c_float) -> c_int;
+    pub fn ssq_issq_cwt_components_batch_f32(ctx: *mut SsqCtx, d_tx: *const c_float, channels: i64, ns: i64, n: i64, wavelet: c_int, scales: *const c_double, d_cc: *const i32, d_cw: *const i32, k: c_int, d_x: *mut c_float) -> c_int;
     pub fn ssq_wavelet_morlet(kind: c_int, w: *const c_double, n: i64, scale: c_double, mu: c_double, out: *mut c_double) -> c_int;
     pub fn ssq_wavelet_gmw(kind: c_int, w: *const c_double, n: i64, scale: c_double, gamma: c_double, beta: c_double, norm_bandpass: c_int, order: c_int, out: *mut c_double) -> c_int;
     pub fn ssq_wavelet_gmw_center_frequency(gamma: c_double, beta: c_double, kind: c_int, out: *mut c_double) -> c_int;

@@ -5,7 +5,7 @@
 // the build image has no Rust toolchain): ssqueeze_rs_b200/_rs.py.
 use ndarray::{Array1, Array2};
 use num_complex::Complex64;
-use numpy::{IntoPyArray, PyReadonlyArray1, PyReadonlyArray2};
+use numpy::{AllowTypeChange, IntoPyArray, PyArrayLikeDyn, PyReadonlyArray1, PyReadonlyArray2};
 use pyo3::exceptions::PyValueError;
 use pyo3::prelude::*;
 use std::os::raw::c_int;
@@ -197,9 +197,32 @@ pub fn istft<'py>(
     Ok(out.into_pyarray(py).into_py(py))
 }
 
-/// Inverse synchrosqueezed STFT (old/ssqueezepy/_ssq_stft.py:139-198; hop_len must be 1, Tx from modulated=True)
+type Bands<'py> = Option<PyArrayLikeDyn<'py, i32, AllowTypeChange>>;
+
+/// cc / cw of the component inversions (old/ssqueezepy/_ssq_cwt.py:380-402): int arrays [n] (one band) or [n, K], each
+/// read as int32 [n][K]; None when neither is given.  Errors are raised before any device work.
+fn bands(cc: Bands<'_>, cw: Bands<'_>, n: usize) -> PyResult<Option<(Vec<i32>, Vec<i32>, usize)>> {
+    let (cc, cw) = match (cc, cw) {
+        (None, None) => return Ok(None),
+        (Some(cc), Some(cw)) => (cc, cw),
+        _ => return Err(PyValueError::new_err("cc and cw go together")),
+    };
+    let (a, b) = (cc.as_array(), cw.as_array());
+    if n == 0 || a.len() % n != 0 || b.len() % n != 0 {
+        return Err(PyValueError::new_err(format!("cannot reshape cc / cw of {} / {} elements to [{n}, K]", a.len(), b.len())));
+    }
+    if a.len() != b.len() {
+        return Err(PyValueError::new_err("cc and cw must have the same shape"));
+    }
+    let k = a.len() / n;
+    Ok(Some((a.iter().copied().collect(), b.iter().copied().collect(), k)))
+}
+
+/// Inverse synchrosqueezed STFT (old/ssqueezepy/_ssq_stft.py:139-198; hop_len must be 1, Tx from modulated=True).
+/// With `cc`, `cw`: the curve bands over the frequency rows, [K + 1, n_frames], the residual last.
 #[pyfunction]
-#[pyo3(signature = (tx, window, n_fft=None, win_len=None, hop_len=1, fs=1.0))]
+#[pyo3(signature = (tx, window, n_fft=None, win_len=None, hop_len=1, fs=1.0, *, cc=None, cw=None))]
+#[allow(clippy::too_many_arguments)]
 pub fn issq_stft<'py>(
     py: Python<'py>,
     tx: PyReadonlyArray2<Complex64>,
@@ -208,12 +231,26 @@ pub fn issq_stft<'py>(
     win_len: Option<usize>,
     hop_len: usize,
     fs: f64,
+    cc: Bands<'py>,
+    cw: Bands<'py>,
 ) -> PyResult<PyObject> {
     let _ = win_len;
     let t = tx.as_array().as_standard_layout().to_owned();
     let w_s = window.as_array().to_owned();
     let (nfq, nfr) = (t.shape()[0], t.shape()[1]);
     let n_fft = n_fft.unwrap_or((nfq - 1) * 2);
+    if let Some((cc, cw, k)) = bands(cc, cw, nfr)? {
+        let mut y = Array2::<f64>::zeros((k + 1, nfr));
+        let st = py.allow_threads(|| {
+            ffi::with_ctx(|c| unsafe {
+                ffi::ssq_issq_stft_components_f64(c, t.as_ptr() as *const f64, nfq as i64, nfr as i64, w_s.as_ptr(),
+                                                  w_s.len() as i64, n_fft as c_int, hop_len as c_int, fs, cc.as_ptr(),
+                                                  cw.as_ptr(), k as c_int, y.as_mut_ptr())
+            })
+        });
+        ffi::with_ctx(|c| ffi::check(st, c))?;
+        return Ok(y.into_pyarray(py).into_py(py));
+    }
     let mut y = Array1::<f64>::zeros(nfr);
     let st = py.allow_threads(|| {
         ffi::with_ctx(|c| unsafe {
@@ -384,11 +421,13 @@ pub fn icwt<'py>(
     Ok(x.into_pyarray(py).into_py(py))
 }
 
-/// Inversion of `ssq_cwt` (spec old/ssqueezepy/_ssq_cwt.py:313-378; full inversion)
+/// Inversion of `ssq_cwt` (spec old/ssqueezepy/_ssq_cwt.py:313-402): the full inversion, or with `cc`, `cw` the curve
+/// bands, [K + 1, n] with the residual last
 #[pyfunction]
-#[pyo3(signature = (tx, wavelet="gmw", scales=None))]
+#[pyo3(signature = (tx, wavelet="gmw", scales=None, cc=None, cw=None))]
 pub fn issq_cwt<'py>(
     py: Python<'py>, tx: PyReadonlyArray2<Complex64>, wavelet: &str, scales: Option<PyReadonlyArray1<f64>>,
+    cc: Bands<'py>, cw: Bands<'py>,
 ) -> PyResult<PyObject> {
     let sc = match scales {
         Some(s) => s.as_array().to_vec(),
@@ -396,8 +435,19 @@ pub fn issq_cwt<'py>(
     };
     let t = tx.as_array().as_standard_layout().to_owned();
     let (ns, n) = (t.shape()[0], t.shape()[1]);
-    let mut x = Array1::<f64>::zeros(n);
     let wav = wavelet_code(wavelet);
+    if let Some((cc, cw, k)) = bands(cc, cw, n)? {
+        let mut x = Array2::<f64>::zeros((k + 1, n));
+        let st = py.allow_threads(|| {
+            ffi::with_ctx(|c| unsafe {
+                ffi::ssq_issq_cwt_components_f64(c, t.as_ptr() as *const f64, ns as i64, n as i64, wav, sc.as_ptr(),
+                                                 cc.as_ptr(), cw.as_ptr(), k as c_int, x.as_mut_ptr())
+            })
+        });
+        ffi::with_ctx(|c| ffi::check(st, c))?;
+        return Ok(x.into_pyarray(py).into_py(py));
+    }
+    let mut x = Array1::<f64>::zeros(n);
     let st = py.allow_threads(|| {
         ffi::with_ctx(|c| unsafe {
             ffi::ssq_issq_cwt_f64(c, t.as_ptr() as *const f64, ns as i64, n as i64, wav, sc.as_ptr(), x.as_mut_ptr())

@@ -65,6 +65,12 @@ SIGNATURES = {
     "ssq_issq_cwt_f64": (c_int, [c_vp, c_vp, c_i64, c_i64, c_int, c_vp, c_vp]),
     "ssq_issq_cwt_components_f64": (c_int, [c_vp, c_vp, c_i64, c_i64, c_int, c_vp, c_vp, c_vp, c_int, c_vp]),
     "ssq_issq_cwt_batch_f32": (c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_int, c_vp, c_vp]),
+    "ssq_issq_cwt_components_batch_f32": (c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_int, c_vp, c_vp, c_vp, c_int,
+                                                  c_vp]),
+    "ssq_issq_stft_components_f64": (c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_int, c_int, c_dbl, c_vp, c_vp,
+                                             c_int, c_vp]),
+    "ssq_issq_stft_components_batch_f32": (c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_int, c_dbl, c_vp,
+                                                   c_vp, c_int, c_vp]),
     "ssq_icwt_batch_f32": (c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_int, c_vp, c_int, c_i64, c_dbl, c_u32, c_vp]),
     "ssq_ssq_stft_batch_f32": (c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_int, c_int, c_dbl,
                                        c_int, c_int, c_dbl, c_u32, c_vp]),

@@ -317,15 +317,36 @@ def istft(Sx, window, n_fft=None, win_len=None, hop_len=1, N=None, win_exp=1):
     return x
 
 
-def issq_stft(Tx, window, n_fft=None, win_len=None, hop_len=1, fs=1.0):
-    """Inverse synchrosqueezed STFT (old/ssqueezepy/_ssq_stft.py:139-198, full
-    inverse).  Needs hop_len == 1 and a Tx computed with `modulated=True`."""
+def _bands(cc, cw, n):
+    """cc, cw (int arrays [n] or [n, K]) -> contiguous int32 [n, K] each, and K."""
+    if (cc is None) != (cw is None):
+        raise ValueError("cc and cw go together")
+    cc = np.ascontiguousarray(np.asarray(cc).reshape(n, -1), dtype=np.int32)
+    cw = np.ascontiguousarray(np.asarray(cw).reshape(n, -1), dtype=np.int32)
+    if cc.shape != cw.shape:
+        raise ValueError("cc and cw must have the same shape")
+    return cc, cw, cc.shape[1]
+
+
+def issq_stft(Tx, window, n_fft=None, win_len=None, hop_len=1, fs=1.0, *, cc=None, cw=None):
+    """Inverse synchrosqueezed STFT (old/ssqueezepy/_ssq_stft.py:139-198).
+    Needs hop_len == 1 and a Tx computed with `modulated=True`.  Without `cc` / `cw`: the full inverse, float64
+    [n_frames].  With them (int arrays [n_frames] or [n_frames, K] as for `issq_cwt`): the curve bands over the
+    frequency rows, [K + 1, n_frames], the last row being the residual."""
     if not isinstance(Tx, np.ndarray) or Tx.ndim != 2 or Tx.dtype != np.complex128:
         raise TypeError("argument 'Tx': expected a 2-D numpy.ndarray of complex128")
     window = _f64_1d(window, "window")
     Tx = np.ascontiguousarray(Tx)
     nfq, nfr = Tx.shape
     nf = int(n_fft) if n_fft else (nfq - 1) * 2
+    if cc is not None or cw is not None:
+        cc, cw, K = _bands(cc, cw, nfr)
+        ctx = default_context()
+        y = np.empty((K + 1, nfr), dtype=np.float64)
+        st = load().ssq_issq_stft_components_f64(ctx.handle, _ptr(Tx), nfq, nfr, _ptr(window), len(window), nf,
+                                                 int(hop_len), float(fs), _ptr(cc), _ptr(cw), K, _ptr(y))
+        raise_status(st, ctx.handle)
+        return y
     ctx = default_context()
     y = np.empty(nfr, dtype=np.float64)
     st = load().ssq_issq_stft_f64(ctx.handle, _ptr(Tx), nfq, nfr, _ptr(window), len(window), nf, int(hop_len),
@@ -479,14 +500,8 @@ def issq_cwt(Tx, wavelet="gmw", scales=None, cc=None, cw=None):
     ns, n = Tx.shape
     ctx = default_context()
     wid = 1 if _str(wavelet, "wavelet") == "morlet" else 0
-    if (cc is None) != (cw is None):
-        raise ValueError("cc and cw go together")
-    if cc is not None:
-        cc = np.ascontiguousarray(np.asarray(cc).reshape(n, -1), dtype=np.int32)
-        cw = np.ascontiguousarray(np.asarray(cw).reshape(n, -1), dtype=np.int32)
-        if cc.shape != cw.shape:
-            raise ValueError("cc and cw must have the same shape")
-        K = cc.shape[1]
+    if cc is not None or cw is not None:
+        cc, cw, K = _bands(cc, cw, n)
         x = np.empty((K + 1, n), dtype=np.float64)
         st = load().ssq_issq_cwt_components_f64(ctx.handle, _ptr(Tx), ns, n, wid, _ptr(sc), _ptr(cc), _ptr(cw), K,
                                                 _ptr(x))

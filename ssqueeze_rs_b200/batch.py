@@ -23,6 +23,35 @@ def _wptr(window):
     return w, C.c_void_p(w.ctypes.data)
 
 
+def _bands(cc, cw, ch, n, device):
+    """cc, cw of the component inversions -> contiguous int32 CUDA tensors [ch, n, K] and K.  cc: int32 CUDA tensor
+    [ch, n, K] (what `Engine.extract_ridges` returns) or [ch, n] (one band); cw: a tensor of the same shape, or an int
+    broadcast to it.  Raises ValueError before anything is launched."""
+    import numbers
+
+    import torch
+    if cc is None or cw is None:
+        raise ValueError("cc and cw go together")
+    if not (isinstance(cc, torch.Tensor) and cc.dtype == torch.int32 and cc.device == device):
+        raise ValueError(f"cc must be an int32 tensor on {device}")
+    if cc.dim() == 2:
+        cc = cc.unsqueeze(-1)
+    if cc.dim() != 3 or tuple(cc.shape[:2]) != (ch, n):
+        raise ValueError(f"cc has shape {tuple(cc.shape)}; expected [{ch}, {n}, K] or [{ch}, {n}]")
+    if isinstance(cw, numbers.Integral) and not isinstance(cw, bool):
+        if not -2**31 <= int(cw) < 2**31:
+            raise ValueError("cw does not fit int32")
+        cw = torch.full_like(cc, int(cw))
+    elif isinstance(cw, torch.Tensor) and cw.dtype == torch.int32 and cw.device == device:
+        if cw.dim() == 2:
+            cw = cw.unsqueeze(-1)
+        if cw.shape != cc.shape:
+            raise ValueError(f"cw has shape {tuple(cw.shape)}, cc {tuple(cc.shape)}")
+    else:
+        raise ValueError(f"cw must be an int or an int32 tensor on {device}")
+    return cc.contiguous(), cw.contiguous(), cc.shape[2]
+
+
 class Engine:
     def __init__(self, device: int = 0):
         self.ctx = Context(device)
@@ -127,10 +156,23 @@ class Engine:
         self.istft_ptr(Sx.data_ptr(), ch, nfq, nfr, window, n_fft, hop_len, n_out, out.data_ptr(), win_exp)
         return out
 
-    def issq_stft(self, Tx, window, n_fft, fs=1.0):
+    def issq_stft(self, Tx, window, n_fft, fs=1.0, cc=None, cw=None):
+        """Tx: complex64 CUDA [channels, n_freqs, n_frames] (hop 1, modulated) -> y float32 [channels, n_frames].
+        With `cc`, `cw` (see `issq_cwt`): the curve bands over the frequency rows, float32 [channels, K + 1, n_frames],
+        row K the residual."""
         import torch
         assert Tx.is_cuda and Tx.dtype == torch.complex64 and Tx.dim() == 3 and Tx.is_contiguous()
         ch, nfq, nfr = Tx.shape
+        if cc is not None or cw is not None:
+            cc, cw, K = _bands(cc, cw, ch, nfr, Tx.device)
+            y = torch.empty((ch, K + 1, nfr), dtype=torch.float32, device=Tx.device)
+            w, wp = _wptr(window)
+            self._bind_stream()
+            st = load().ssq_issq_stft_components_batch_f32(self.ctx.handle, C.c_void_p(Tx.data_ptr()), ch, nfq, nfr, wp,
+                                                           len(w), int(n_fft), float(fs), C.c_void_p(cc.data_ptr()),
+                                                           C.c_void_p(cw.data_ptr()), K, C.c_void_p(y.data_ptr()))
+            raise_status(st, self.ctx.handle)
+            return y
         out = torch.empty((ch, nfr), dtype=torch.float32, device=Tx.device)
         self._bind_stream()
         self.issq_stft_ptr(Tx.data_ptr(), ch, nfq, nfr, window, n_fft, fs, out.data_ptr())
@@ -214,12 +256,27 @@ class Engine:
         raise_status(st, self.ctx.handle)
         return x
 
-    def issq_cwt(self, Tx, scales, wavelet="gmw"):
-        """Tx: complex64 CUDA [channels, ns, n] -> x float32 [channels, n] (full inversion)."""
+    def issq_cwt(self, Tx, scales, wavelet="gmw", cc=None, cw=None):
+        """Tx: complex64 CUDA [channels, ns, n] -> x float32 [channels, n] (full inversion).
+        With `cc`, `cw`: the component inversion (old/ssqueezepy/_ssq_cwt.py:380-402) of K curve bands, float32
+        [channels, K + 1, n], row K the residual.  cc: int32 CUDA tensor [channels, n, K] of centre rows, e.g. the
+        indices `extract_ridges` returns (cc == -1: no curve at that column), or [channels, n] for one band; cw: the
+        half-widths, a tensor of the same shape or an int.  Band c of column j is the rows clip(cc - cw, 0, ns) ..
+        clip(cc + cw, 0, ns), clipped on the device; 1 <= K <= 16."""
         import torch
         assert Tx.is_cuda and Tx.dtype == torch.complex64 and Tx.dim() == 3 and Tx.is_contiguous()
         ch, ns, n = Tx.shape
         sc = np.ascontiguousarray(scales, dtype=np.float64)
+        if cc is not None or cw is not None:
+            cc, cw, K = _bands(cc, cw, ch, n, Tx.device)
+            x = torch.empty((ch, K + 1, n), dtype=torch.float32, device=Tx.device)
+            self._bind_stream()
+            st = load().ssq_issq_cwt_components_batch_f32(self.ctx.handle, C.c_void_p(Tx.data_ptr()), ch, ns, n,
+                                                          1 if wavelet == "morlet" else 0, C.c_void_p(sc.ctypes.data),
+                                                          C.c_void_p(cc.data_ptr()), C.c_void_p(cw.data_ptr()), K,
+                                                          C.c_void_p(x.data_ptr()))
+            raise_status(st, self.ctx.handle)
+            return x
         x = torch.empty((ch, n), dtype=torch.float32, device=Tx.device)
         self._bind_stream()
         st = load().ssq_issq_cwt_batch_f32(self.ctx.handle, C.c_void_p(Tx.data_ptr()), ch, ns, n,

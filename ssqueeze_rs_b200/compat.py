@@ -138,17 +138,33 @@ def istft(Sx, window=None, n_fft=None, win_len=None, hop_len=1, N=None, modulate
 
 
 def issq_stft(Tx, window=None, cc=None, cw=None, n_fft=None, win_len=None, hop_len=1, modulated=True):
-    """old/ssqueezepy/_ssq_stft.py:139-198 (full inversion; `cc` / `cw` are not supported here)."""
+    """old/ssqueezepy/_ssq_stft.py:139-198.  Without `cc` / `cw` the full inversion, [n_frames]; with them the curve
+    bands of `_invert_components` (_ssq_cwt.py:380-402) times upstream's 2 / window[n_fft // 2], [K + 1, n_frames]
+    with the residual last.  1-D cc / cw are one band, as upstream's reshape(-1, 1)."""
     if not modulated:
         raise ValueError("inversion with `modulated == False` is unsupported.")
     if hop_len != 1:
         raise ValueError("inversion with `hop_len != 1` is unsupported.")
-    if cc is not None or cw is not None:
-        raise NotImplementedError("compat.issq_stft: component inversion")
+    if (cc is None) != (cw is None):
+        raise ValueError("cc and cw go together")
     Tx = np.ascontiguousarray(Tx, dtype=np.complex128)
     nfq, nfr = Tx.shape
     n_fft = n_fft or (nfq - 1) * 2
     win_len = win_len or n_fft
+    if cc is not None:
+        cc, cw = np.asarray(cc), np.asarray(cw)
+        cc, cw = (cc.reshape(-1, 1) if cc.ndim == 1 else cc), (cw.reshape(-1, 1) if cw.ndim == 1 else cw)
+        if cc.ndim != 2 or cc.shape != cw.shape or cc.shape[0] != nfr:
+            raise ValueError(f"cc {cc.shape} and cw {cw.shape} must both be [n_frames = {nfr}, K]")
+        cc = np.ascontiguousarray(cc, dtype=np.int32)
+        cw = np.ascontiguousarray(cw, dtype=np.int32)
+        w = get_window(window, int(win_len), int(n_fft))
+        ctx = _context()
+        y = np.empty((cc.shape[1] + 1, nfr), dtype=np.float64)
+        st = load().ssq_issq_stft_components_f64(ctx.handle, _ptr(Tx), nfq, nfr, _ptr(w), len(w), int(n_fft), 1, 1.0,
+                                                 _ptr(cc), _ptr(cw), cc.shape[1], _ptr(y))
+        raise_status(st, ctx.handle)
+        return y
     w = get_window(window, int(win_len), int(n_fft))
     ctx = _context()
     y = np.empty(nfr, dtype=np.float64)

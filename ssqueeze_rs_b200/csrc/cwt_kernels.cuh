@@ -687,45 +687,6 @@ __global__ void icwt_kernel(const float2* __restrict__ Wx, int64_t ns, int64_t n
 }
 
 // ------------------------------------------------------------------------------------
-// issq_cwt, component inversion (old/ssqueezepy/_ssq_cwt.py:380-402): component c of column j sums
-// Re Tx[k][j] over the rows lo[j][c] <= k <= hi[j][c] (each component from the ORIGINAL Tx, so bands
-// may overlap); the residual is the sum over the rows no band covers.  One thread per column,
-// rows in ascending order, Tx read once.  x: [K + 1][n].
-// ------------------------------------------------------------------------------------
-#define SSQ_MAX_COMPONENTS 16
-__global__ void issq_cwt_components_kernel(const float2* __restrict__ Tx, int ns, int64_t n, int K,
-                                           const int* __restrict__ lo, const int* __restrict__ hi, float scale,
-                                           float* __restrict__ x) {
-  const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (j >= n) return;
-  int l[SSQ_MAX_COMPONENTS], h[SSQ_MAX_COMPONENTS];
-  float acc[SSQ_MAX_COMPONENTS + 1];
-#pragma unroll
-  for (int c = 0; c < SSQ_MAX_COMPONENTS; ++c) {
-    l[c] = c < K ? lo[j * K + c] : 1;
-    h[c] = c < K ? hi[j * K + c] : 0;
-    acc[c] = 0.f;
-  }
-  float rest = 0.f;
-  for (int k = 0; k < ns; ++k) {
-    const float v = __ldcs(Tx + (size_t)k * n + j).x;
-    bool covered = false;
-#pragma unroll
-    for (int c = 0; c < SSQ_MAX_COMPONENTS; ++c) {
-      if (k >= l[c] && k <= h[c]) {
-        acc[c] += v;
-        covered = true;
-      }
-    }
-    if (!covered) rest += v;
-  }
-#pragma unroll
-  for (int c = 0; c < SSQ_MAX_COMPONENTS; ++c)
-    if (c < K) x[(size_t)c * n + j] = acc[c] * scale;
-  x[(size_t)K * n + j] = rest * scale;
-}
-
-// ------------------------------------------------------------------------------------
 // icwt, two-integral branch (cwt.rs:629-712) in the frequency domain:
 //   S[k] = sum_i FFT(Wx[i])[k] * psi-hat(scale_i xi_k) / scale_i   (psi-hat real; peak-normalised here, the constant
 //   goes into the final factor), then x = Re(IFFT(S)) * norm + x_mean.

@@ -13,6 +13,7 @@
 #include "istft_r256.cuh"
 #include "istream_kernels.cuh"
 #include "cwt_kernels.cuh"
+#include "components_kernels.cuh"
 #include "ridge_kernels.cuh"
 
 #include <algorithm>
@@ -29,8 +30,8 @@ static const double kEps64 = 2.2204460492503131e-16;
 // library / context
 // ===========================================================================
 extern "C" const char* ssq_version(void) {
-  return "ssqcuda 0.3 (B200 sm_100a; stft, ssq_stft, istft, issq_stft, cwt, cwt_simd, ssq_cwt, icwt, issq_cwt, "
-         "ssq_stft streaming, istft / issq_stft streaming, ridge extraction)";
+  return "ssqcuda 0.4 (B200 sm_100a; stft, ssq_stft, istft, issq_stft, cwt, cwt_simd, ssq_cwt, icwt, issq_cwt, "
+         "ssq_stft streaming, istft / issq_stft streaming, ridge extraction, issq_cwt / issq_stft components)";
 }
 
 // lib.rs:16-19
@@ -660,6 +661,32 @@ extern "C" ssq_status ssq_issq_stft_batch_f32(ssq_ctx* ctx, const float* d_Tx, i
   return SSQ_OK;
 }
 
+// issq_stft with curve bands: the component inversion of issq_components_kernel (components_kernels.cuh) on a hop-1,
+// modulated Tx, times the factor of ssq_issq_stft_batch_f32.  The arguments are checked before the context.
+extern "C" ssq_status ssq_issq_stft_components_batch_f32(ssq_ctx* ctx, const float* d_Tx, int64_t channels,
+                                                         int64_t n_freqs, int64_t n_frames, const double* window,
+                                                         int64_t win_n, int n_fft, double fs, const int32_t* d_cc,
+                                                         const int32_t* d_cw, int K, float* d_y) {
+  if (K < 1 || K > SSQ_MAX_COMPONENTS)
+    return ssq_fail(ctx, SSQ_EUNSUPPORTED, "issq_stft: %d components (1..%d supported)", K, SSQ_MAX_COMPONENTS);
+  if (!ctx) return ssq_fail(nullptr, SSQ_EINVAL, "ctx is NULL");
+  if (!d_Tx || !d_y || !d_cc || !d_cw || !window || win_n < 1) return ssq_fail(ctx, SSQ_EINVAL, "NULL/empty argument");
+  if (n_fft <= 0) n_fft = (int)(n_freqs - 1) * 2;
+  if (n_fft < 2 || n_fft / 2 + 1 != n_freqs)
+    return ssq_fail(ctx, SSQ_EINVAL, "Tx has %lld rows but n_fft=%d needs %d", (long long)n_freqs, n_fft,
+                    n_fft / 2 + 1);
+  if (n_frames < 1 || channels < 1) return ssq_fail(ctx, SSQ_EINVAL, "empty Tx");
+  if (channels > 65535) return ssq_fail(ctx, SSQ_EUNSUPPORTED, "issq_stft: %lld channels in one call", (long long)channels);
+  SSQ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  std::vector<double> wfit = ssqhost::fit_window(window, win_n, n_fft);
+  const float scale = (float)(2.0 / (wfit[(size_t)(n_fft / 2)] * fs));
+  SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+  SSQ_TRY(issq_components_run(ctx, (const float2*)d_Tx, channels, n_freqs, n_frames, d_cc, d_cw, K, scale, d_y));
+  SSQ_CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+  ctx->ev_valid = true;
+  return SSQ_OK;
+}
+
 // ---------------------------------------------------------------------------
 // reference-typed entry points (host f64 / c128)
 // ---------------------------------------------------------------------------
@@ -859,6 +886,29 @@ extern "C" ssq_status ssq_issq_stft_f64(ssq_ctx* ctx, const double* Tx, int64_t 
   SSQ_TRY(ssq_issq_stft_batch_f32(ctx, (const float*)ctx->ws_in.p, 1, n_freqs, n_frames, window, win_n, n_fft, fs,
                                   (float*)ctx->ws_out.p));
   return download_f32_as_f64(ctx, ctx->ws_out.p, (size_t)n_frames, y);
+}
+
+extern "C" ssq_status ssq_issq_stft_components_f64(ssq_ctx* ctx, const double* Tx, int64_t n_freqs, int64_t n_frames,
+                                                   const double* window, int64_t win_n, int n_fft, int hop, double fs,
+                                                   const int32_t* cc, const int32_t* cw, int K, double* y) {
+  if (K < 1 || K > SSQ_MAX_COMPONENTS)
+    return ssq_fail(ctx, SSQ_EUNSUPPORTED, "issq_stft: %d components (1..%d supported)", K, SSQ_MAX_COMPONENTS);
+  if (!ctx) return ssq_fail(nullptr, SSQ_EINVAL, "ctx is NULL");
+  if (!Tx || !window || !y || !cc || !cw) return ssq_fail(ctx, SSQ_EINVAL, "NULL argument");
+  if (hop != 1) return ssq_fail(ctx, SSQ_EINVAL, "inversion with `hop_len != 1` is unsupported.");
+  if (n_freqs < 2 || n_frames < 1) return ssq_fail(ctx, SSQ_EINVAL, "bad Tx shape");
+  SSQ_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  const size_t cnt = (size_t)n_freqs * n_frames, nb = (size_t)n_frames * K;
+  SSQ_TRY(upload_f64_as_f32(ctx, Tx, cnt * 2, ctx->ws_in));
+  SSQ_TRY(devbuf_reserve(ctx, ctx->ws_aux0, 2 * nb * sizeof(int32_t)));
+  SSQ_TRY(devbuf_reserve(ctx, ctx->ws_out, (size_t)(K + 1) * n_frames * sizeof(float)));
+  int32_t* d_cc = (int32_t*)ctx->ws_aux0.p;
+  int32_t* d_cw = d_cc + nb;
+  SSQ_CUDA_TRY(ctx, cudaMemcpyAsync(d_cc, cc, nb * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+  SSQ_CUDA_TRY(ctx, cudaMemcpyAsync(d_cw, cw, nb * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+  SSQ_TRY(ssq_issq_stft_components_batch_f32(ctx, (const float*)ctx->ws_in.p, 1, n_freqs, n_frames, window, win_n,
+                                             n_fft, fs, d_cc, d_cw, K, (float*)ctx->ws_out.p));
+  return download_f32_as_f64(ctx, ctx->ws_out.p, (size_t)(K + 1) * n_frames, y);
 }
 
 // ---------------------------------------------------------------------------
