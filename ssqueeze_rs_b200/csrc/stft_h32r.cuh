@@ -1,5 +1,5 @@
-// stft_h32r.cuh -- "rotated" variant of the n_fft = 512 kernel (hop = 32: register sliding window; any
-// other hop: per-frame reload): the item staging
+// stft_h32r.cuh -- "rotated" variant of the n_fft = 512 kernel (hop = 32: sliding sample window, in tensor memory in
+// the ssq mode; any other hop: per-frame reload): the item staging
 // (transposition of the 257 (bin, value) items through shared memory: 48 wavefronts per
 // frame on the binding L1TEX data pipe) is removed.
 //
@@ -225,7 +225,68 @@ __device__ __noinline__ float h32r_edge_sample(const float* x, int64_t n, int64_
 // and needs the 256 B segments of 32-frame tiles at full scale (384 channels: 18.1 vs 26.5 ms).
 #define H32R_NW(MODE) ((MODE) == 1 ? 8 : 4)
 
-// SLIDE: hop == 32, the register sliding window (one new sample per lane and frame).  Otherwise any hop:
+// Tensor memory (TMEM) of the ssq mode: warp w uses lane quarter w (lanes 32w..32w+31), one lane per thread.
+// Columns 0..31 hold the lane's window taps, (w, dw*s) at positions lane + 32 j, j = 0..15, in column
+// 4t + {0, 1, 2, 3} = (w, dw*s)[lane + 64 t], (w, dw*s)[lane + 32 + 64 t].  At hop 32, columns 32..50 hold the samples of
+// the warp's tile: sample lane + 32 b of its first frame in column 32 + b, so frame s of the tile reads its 16 samples
+// from columns 32 + s .. 47 + s.  Read by tcgen05.ld (LDTM), which does not go through the L1TEX data pipe that binds
+// this kernel (profiles/README.md, round 3): 32 shared wavefronts per frame fewer than the shared tap table, and the
+// 16-register sample window is no longer live across the FFT and the reassignment.
+
+__device__ __forceinline__ void h32r_tmem_st32(uint32_t taddr, const float (&v)[32]) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,"
+      "%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31,%32};\n\t"
+      "tcgen05.wait::st.sync.aligned;" ::"r"(taddr),
+      "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]), "f"(v[8]), "f"(v[9]),
+      "f"(v[10]), "f"(v[11]), "f"(v[12]), "f"(v[13]), "f"(v[14]), "f"(v[15]), "f"(v[16]), "f"(v[17]), "f"(v[18]),
+      "f"(v[19]), "f"(v[20]), "f"(v[21]), "f"(v[22]), "f"(v[23]), "f"(v[24]), "f"(v[25]), "f"(v[26]), "f"(v[27]),
+      "f"(v[28]), "f"(v[29]), "f"(v[30]), "f"(v[31]));
+}
+
+__device__ __forceinline__ void h32r_tmem_st16(uint32_t taddr, const float (&v)[17]) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr),
+      "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]), "f"(v[8]), "f"(v[9]),
+      "f"(v[10]), "f"(v[11]), "f"(v[12]), "f"(v[13]), "f"(v[14]), "f"(v[15]));
+}
+
+__device__ __forceinline__ void h32r_tmem_st1(uint32_t taddr, float v) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x1.b32 [%0], {%1};" ::"r"(taddr), "f"(v));
+}
+
+// the frame's 16 samples and the 32 taps: waits for this thread's earlier sample stores, loads, waits for the loads
+__device__ __forceinline__ void h32r_tmem_ld_window(uint32_t taddr_x, uint32_t taddr_w, float (&x)[16], float (&v)[32]) {
+  asm volatile(
+      "tcgen05.wait::st.sync.aligned;\n\t"
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%48];\n\t"
+      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31,%32,%33,"
+      "%34,%35,%36,%37,%38,%39,%40,%41,%42,%43,%44,%45,%46,%47}, [%49];\n\t"
+      "tcgen05.wait::ld.sync.aligned;"
+      : "=f"(x[0]), "=f"(x[1]), "=f"(x[2]), "=f"(x[3]), "=f"(x[4]), "=f"(x[5]), "=f"(x[6]), "=f"(x[7]), "=f"(x[8]),
+        "=f"(x[9]), "=f"(x[10]), "=f"(x[11]), "=f"(x[12]), "=f"(x[13]), "=f"(x[14]), "=f"(x[15]),
+        "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7]), "=f"(v[8]),
+        "=f"(v[9]), "=f"(v[10]), "=f"(v[11]), "=f"(v[12]), "=f"(v[13]), "=f"(v[14]), "=f"(v[15]), "=f"(v[16]),
+        "=f"(v[17]), "=f"(v[18]), "=f"(v[19]), "=f"(v[20]), "=f"(v[21]), "=f"(v[22]), "=f"(v[23]), "=f"(v[24]),
+        "=f"(v[25]), "=f"(v[26]), "=f"(v[27]), "=f"(v[28]), "=f"(v[29]), "=f"(v[30]), "=f"(v[31])
+      : "r"(taddr_x), "r"(taddr_w));
+}
+
+// load and wait in one statement: the values exist for the compiler only once the wait is done
+__device__ __forceinline__ void h32r_tmem_ld32(uint32_t taddr, float (&v)[32]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,"
+      "%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];\n\t"
+      "tcgen05.wait::ld.sync.aligned;"
+      : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7]), "=f"(v[8]),
+        "=f"(v[9]), "=f"(v[10]), "=f"(v[11]), "=f"(v[12]), "=f"(v[13]), "=f"(v[14]), "=f"(v[15]), "=f"(v[16]),
+        "=f"(v[17]), "=f"(v[18]), "=f"(v[19]), "=f"(v[20]), "=f"(v[21]), "=f"(v[22]), "=f"(v[23]), "=f"(v[24]),
+        "=f"(v[25]), "=f"(v[26]), "=f"(v[27]), "=f"(v[28]), "=f"(v[29]), "=f"(v[30]), "=f"(v[31])
+      : "r"(taddr));
+}
+
+// SLIDE: hop == 32, the sliding window (one new sample per lane and frame; in TMEM in the ssq mode, in registers in the
+// stft mode).  Otherwise any hop:
 // the 16 samples of every frame are (re)loaded, still a whole frame ahead of their use.
 template <int MODE, int SQZ, bool SLIDE, bool DBG = false>
 __global__ void __launch_bounds__(H32R_NW(MODE) * 32, 16 / H32R_NW(MODE)) ssq_stft512_h32r_kernel(const StftParams P) {
@@ -233,14 +294,28 @@ __global__ void __launch_bounds__(H32R_NW(MODE) * 32, 16 / H32R_NW(MODE)) ssq_st
   // stft at hop 32: two frames per FFT (z = x_A w + i x_B w; frame B's samples are frame A's window
   // shifted by one position), so a warp runs 2 FFTs for its 4 frames
   constexpr bool PAIR = (MODE == 1) && SLIDE;
+  // the window taps: a shared table in the stft mode, tensor memory in the ssq mode; at hop 32 the ssq mode's sample
+  // window too (RING)
+  constexpr bool TM = MODE == 0;
+  constexpr bool RING = TM && SLIDE;
+  constexpr int TMC = RING ? 64 : 32;  // TMEM columns per CTA
+  constexpr int WT = TM ? 0 : N;
   extern __shared__ float2 smem[];
-  float2* wtab = smem;          // [512] (w, dw*s)
-  float2* tw2tab = smem + N;    // [8][9]
-  float2* acc = smem + N + 72;  // [32][AS] the tile's Tx columns
+  __shared__ uint32_t tmem_base_s;
+  float2* wtab = smem;           // [WT] (w, dw*s)
+  float2* tw2tab = smem + WT;    // [8][9]
+  float2* acc = smem + WT + 72;  // [32][AS] the tile's Tx columns
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  float2* xch = acc + F * AS + warp * N;  // 584 + F * 261 float2 is even (F = 16, 32): the float4 exchange rows stay 16 B aligned
+  float2* xch = acc + F * AS + warp * N;  // WT + 72 + F * 261 float2 is even (F = 16, 32): the float4 exchange rows stay 16 B aligned
 
-  for (int i = threadIdx.x; i < N; i += blockDim.x) wtab[i] = make_float2(P.win[i], P.dwin[i]);
+  if (TM && warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
+                     (uint32_t)__cvta_generic_to_shared(&tmem_base_s)),
+                 "n"(TMC));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+  }
+  if (!TM)
+    for (int i = threadIdx.x; i < N; i += blockDim.x) wtab[i] = make_float2(P.win[i], P.dwin[i]);
   if (threadIdx.x < 64)
     tw2tab[(threadIdx.x >> 3) * 9 + (threadIdx.x & 7)] = P.tw[((threadIdx.x >> 3) * (threadIdx.x & 7) * 8) & (N - 1)];
   for (int i = threadIdx.x; i < F * AS; i += blockDim.x) acc[i] = make_float2(0.f, 0.f);
@@ -276,7 +351,22 @@ __global__ void __launch_bounds__(H32R_NW(MODE) * 32, 16 / H32R_NW(MODE)) ssq_st
     skf0 = rho <= 3 ? (float)ka : (float)(ka - 512);
     wrapd = -448.f;
   }
+  if (TM) asm volatile("tcgen05.fence::before_thread_sync;");
   __syncthreads();
+  uint32_t taps = 0;  // this warp's lane quarter of the CTA's TMEM columns (column 0)
+  if (TM) {
+    asm volatile("tcgen05.fence::after_thread_sync;");
+    taps = tmem_base_s + ((uint32_t)(warp * 32) << 16);
+    float v[32];
+#pragma unroll
+    for (int t = 0; t < 8; ++t) {
+      v[4 * t] = P.win[lane + 64 * t];
+      v[4 * t + 1] = P.dwin[lane + 64 * t];
+      v[4 * t + 2] = P.win[lane + 32 + 64 * t];
+      v[4 * t + 3] = P.dwin[lane + 32 + 64 * t];
+    }
+    h32r_tmem_st32(taps, v);  // waits for the store: the frames below load from it
+  }
 
   // ---- the warp's frames of a tile: [f0, f0 + nfr), nfr in 0..4 ------------------------------
   const float* xc = nullptr;
@@ -316,17 +406,35 @@ __global__ void __launch_bounds__(H32R_NW(MODE) * 32, 16 / H32R_NW(MODE)) ssq_st
     const int tnf = real ? (int)min((int64_t)F, P.n_frames - tf0) : 0;
     const int next = tile + (int)gridDim.x;
     const int my_n = real ? nfr : 0;
+    if (RING && real) h32r_tmem_st16(taps + 32, xw);  // the tile's window, loaded during the previous tile's store
 #pragma unroll 1
     for (int s = 0; s < 4; s += (PAIR ? 2 : 1)) {
       const bool active = s < my_n;
       float2 va[8], vb[8];
+      float xn = 0.f;  // RING: the sample this lane adds for frame s + 1
       if (active) {
+        float tv[TM ? 32 : 1];
+        float xs[RING ? 16 : 1];
+        if constexpr (RING)
+          h32r_tmem_ld_window(taps + 32 + s, taps, xs, tv);
+        else if constexpr (TM)
+          h32r_tmem_ld32(taps, tv);
 #pragma unroll
         for (int t = 0; t < 8; ++t) {
-          const float2 w0 = wtab[lane + 64 * t], w1 = wtab[lane + 32 + 64 * t];
+          float2 w0, w1;
+          if constexpr (TM) {
+            w0 = make_float2(tv[4 * t], tv[4 * t + 1]);
+            w1 = make_float2(tv[4 * t + 2], tv[4 * t + 3]);
+          } else {
+            w0 = wtab[lane + 64 * t];
+            w1 = wtab[lane + 32 + 64 * t];
+          }
           if (PAIR) {  // real part frame s, imaginary part frame s+1 (same window, samples one position on)
             va[t] = mul2<false>(make_float2(xw[2 * t], xw[2 * t + 1]), bc2(w0.x));
             vb[t] = mul2<false>(make_float2(xw[2 * t + 1], xw[2 * t + 2]), bc2(w1.x));
+          } else if constexpr (RING) {
+            va[t] = mul2(bc2(xs[2 * t]), w0);
+            vb[t] = mul2(bc2(xs[2 * t + 1]), w1);
           } else {
             va[t] = mul2(bc2(xw[2 * t]), w0);
             vb[t] = mul2(bc2(xw[2 * t + 1]), w1);
@@ -334,7 +442,7 @@ __global__ void __launch_bounds__(H32R_NW(MODE) * 32, 16 / H32R_NW(MODE)) ssq_st
         }
       }
       if (s == (PAIR ? 2 : 3)) {
-        if (next < ntiles) open_tile(next);
+        if (!RING && next < ntiles) open_tile(next);
       } else if (s + (PAIR ? 2 : 1) < my_n) {
         if (PAIR) {
 #pragma unroll
@@ -347,6 +455,9 @@ __global__ void __launch_bounds__(H32R_NW(MODE) * 32, 16 / H32R_NW(MODE)) ssq_st
             xw[15] = h32r_edge_sample(xc, P.n, p, P.left, P.padtype, P.x_origin);
             xw[16] = h32r_edge_sample(xc, P.n, p + 32, P.left, P.padtype, P.x_origin);
           }
+        } else if (RING) {  // a frame ahead of its use; to TMEM after this frame's FFT
+          const int64_t p = (f0 + s + 1) * 32 + lane + 480;
+          xn = inner ? __ldg(xc + (p - lo)) : h32r_edge_sample(xc, P.n, p, P.left, P.padtype, P.x_origin);
         } else if (SLIDE) {
 #pragma unroll
           for (int j = 0; j < 15; ++j) xw[j] = xw[j + 1];
@@ -367,7 +478,10 @@ __global__ void __launch_bounds__(H32R_NW(MODE) * 32, 16 / H32R_NW(MODE)) ssq_st
         h32r_frame<MODE, SQZ, DBG>(P, L, skf0, wrapd, txs, xch, acc + (4 * warp + s) * AS,
                                    PAIR ? acc + (4 * warp + s + 1) * AS : nullptr, va, vb,
                                    DBG ? (size_t)tch * 257 * P.n_frames + tf0 + 4 * warp + s : 0);
+      if (RING && s + 1 < my_n) h32r_tmem_st1(taps + 48 + s, xn);
     }
+    // RING: the next tile's window is fetched here, so that the loads are in flight during the tile store below
+    if (RING && next < ntiles) open_tile(next);
     if (!real) continue;
     __syncthreads();
     // ---- coalesced store: thread -> (frame fr, row group v in 0..7); rows k = v + 8 i live at
@@ -397,6 +511,13 @@ __global__ void __launch_bounds__(H32R_NW(MODE) * 32, 16 / H32R_NW(MODE)) ssq_st
     }
     __syncthreads();
   }
+  if (TM) {  // every warp's last TMEM load is done before the allocating warp frees the columns
+    asm volatile("tcgen05.fence::before_thread_sync;");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;");
+    if (warp == 0)
+      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base_s), "n"(TMC));
+  }
 }
 
 static ssq_status stft_h32r_launch(ssq_ctx* ctx, StftParams& P, bool* done) {
@@ -409,7 +530,8 @@ static ssq_status stft_h32r_launch(ssq_ctx* ctx, StftParams& P, bool* done) {
   P.total_tiles = P.tiles_per_channel * P.channels;
   if (P.total_tiles > (int64_t)0x7ff00000) return SSQ_OK;  // *done stays false: the older kernels index in 64 bits
   *done = true;
-  const size_t smem = ((size_t)512 + 72 + (size_t)F * H32R_AS + (size_t)NW * 512) * sizeof(float2);
+  const size_t wt = P.mode == 1 ? 512 : 0;  // the ssq mode keeps its window taps in tensor memory
+  const size_t smem = (wt + 72 + (size_t)F * H32R_AS + (size_t)NW * 512) * sizeof(float2);
   const int grid = (int)std::min<int64_t>(P.total_tiles, (int64_t)ctx->num_sms * (16 / NW));
   const bool leb = P.squeezing == SSQ_SQUEEZE_LEBESGUE;
   void (*k)(const StftParams);
