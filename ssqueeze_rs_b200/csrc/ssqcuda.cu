@@ -1106,6 +1106,17 @@ extern "C" ssq_status ssq_stream_create_ex(ssq_ctx* ctx, int64_t channels, int64
                       (long long)s->cap, cudaGetErrorString(e));
     }
   }
+  // stft mode pairs frames in one complex FFT: the partner of the last ready frame reads samples not received yet.
+  // Its values only reach the real frame through the rounding of the split, unless they are huge or NaN, which
+  // never-written device memory (freed by an earlier user in this process) can hold.
+  for (int i = 0; i < 2; ++i) {
+    cudaError_t e = cudaMemsetAsync(s->buf[i], 0, (size_t)channels * s->cap * sizeof(float), ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) {
+      ssq_stream_destroy(s);
+      return ssq_fail(ctx, SSQ_ECUDA, "stream buffers: %s", cudaGetErrorString(e));
+    }
+  }
   *out = s;
   return SSQ_OK;
 }
