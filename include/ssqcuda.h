@@ -28,6 +28,9 @@
  *  - streams (`ssq_stream_*` forward, `ssq_istream_*` inverse) take a long
  *    recording chunk by chunk and are exact at chunk seams; they own their
  *    buffers, so calls on the same context between two pushes are allowed;
+ *    the CWT streams (`ssq_stream_create_cwt`) are blockwise with an overlap,
+ *    as the reference's dask caller is, and independent of how the recording
+ *    is cut into pushes;
  *  - there is no CPU fallback: without a usable CUDA device every compute
  *    call fails with SSQ_ECUDA.
  */
@@ -344,6 +347,26 @@ ssq_status ssq_stream_push_i16(ssq_stream* s, const int16_t* d_chunk, int64_t n_
                                float* d_Tx, int64_t* frames_written);
 ssq_status ssq_stream_push_f32(ssq_stream* s, const float* d_chunk, int64_t n_new, float scale,
                                float* d_Tx, int64_t* frames_written);
+
+/* CWT streams (DESIGN §3.6b): the dask map_overlap(depth=overlap, boundary="reflect") caller of the reference's CWT
+ * scripts (tests/cwt_test.py:117-119,187-193), computed on the device from the carry-over buffer.  Block b covers
+ * output columns [b block, min((b + 1) block, n_total)); it is the reference's call (mode 2: cwt -> Wx with
+ * SSQ_FLAG_L2_NORM as in ssq_cwt_batch_f32; mode 3: ssq_cwt -> Tx with SSQ_FLAG_NO_FLIPUD as in
+ * ssq_ssq_cwt_batch_f32) on e_b[j] = x~[b block - overlap + j], j < len_b + 2 overlap, trimmed to columns
+ * [overlap, overlap + len_b); x~ mirrors the recording with the edge sample repeated (np.pad mode "symmetric").  The
+ * scales are the same for every block; maprange maximal uses each block's own length (ssq_stream_ssq_freqs).  A block
+ * is ready once min(n_total, (b + 1) block + overlap) samples have arrived; a push writes every block that became
+ * ready: d_Tx complex64 [channels, ns, cols], cols = ssq_stream_frames_after(s, n_new) queried before the push;
+ * ssq_stream_total_frames is n_total.  The output does not depend on how the recording is cut into pushes.
+ * 1 <= block, 0 <= overlap <= min(block, n_total); the arguments are checked before ctx.  Pushes and the feeder are
+ * those of the STFT streams. */
+ssq_status ssq_stream_create_cwt(ssq_ctx* ctx, int64_t channels, int64_t n_total, int64_t max_chunk, int64_t block,
+                                 int64_t overlap, int mode, int wavelet, const double* scales, int64_t ns, double dt,
+                                 int freq_dist, int padtype, int squeezing, int maprange, double gamma,
+                                 unsigned flags, ssq_stream** out);
+/* the ssq grid of an ssq_cwt stream (float64 [ns]): of the full blocks (last_block = 0) or of the last block, whose
+ * grid differs under maprange maximal when it is shorter */
+ssq_status ssq_stream_ssq_freqs(const ssq_stream* s, int last_block, double* out);
 
 /* Host feeder of a stream: the chunk pointer is HOST memory (pageable is fine: a memory-mapped (samples, channels)
  * .dat / .bin as the reference's scripts read them, tests/stft_ssq_test.py:218-283, tests/stft_test.py:374-377).

@@ -81,6 +81,8 @@ extern "C" {
     pub fn ssq_stream_frames_after(s: *const SsqStream, n_new: i64) -> i64;
     pub fn ssq_stream_push_i16(s: *mut SsqStream, d_chunk: *const i16, n_new: i64, scale: c_float, d_tx: *mut c_float, frames_written: *mut i64) -> c_int;
     pub fn ssq_stream_push_f32(s: *mut SsqStream, d_chunk: *const c_float, n_new: i64, scale: c_float, d_tx: *mut c_float, frames_written: *mut i64) -> c_int;
+    pub fn ssq_stream_create_cwt(ctx: *mut SsqCtx, channels: i64, n_total: i64, max_chunk: i64, block: i64, overlap: i64, mode: c_int, wavelet: c_int, scales: *const c_double, ns: i64, dt: c_double, freq_dist: c_int, padtype: c_int, squeezing: c_int, maprange: c_int, gamma: c_double, flags: c_uint, out: *mut *mut SsqStream) -> c_int;
+    pub fn ssq_stream_ssq_freqs(s: *const SsqStream, last_block: c_int, out: *mut c_double) -> c_int;
     pub fn ssq_feeder_create(s: *mut SsqStream, dtype: c_int, depth: c_int, out: *mut *mut SsqFeeder) -> c_int;
     pub fn ssq_feeder_destroy(f: *mut SsqFeeder);
     pub fn ssq_feeder_push(f: *mut SsqFeeder, h_chunk: *const c_void, n_new: i64, scale: c_float, d_tx: *mut c_float, frames_written: *mut i64) -> c_int;

@@ -103,6 +103,9 @@ SIGNATURES = {
     "ssq_stream_frames_after": (c_i64, [c_vp, c_i64]),
     "ssq_stream_push_i16": (c_int, [c_vp, c_vp, c_i64, C.c_float, c_vp, C.POINTER(c_i64)]),
     "ssq_stream_push_f32": (c_int, [c_vp, c_vp, c_i64, C.c_float, c_vp, C.POINTER(c_i64)]),
+    "ssq_stream_create_cwt": (c_int, [c_vp, c_i64, c_i64, c_i64, c_i64, c_i64, c_int, c_int, c_vp, c_i64, c_dbl,
+                                      c_int, c_int, c_int, c_int, c_dbl, C.c_uint, C.POINTER(c_vp)]),
+    "ssq_stream_ssq_freqs": (c_int, [c_vp, c_int, c_vp]),
     "ssq_feeder_create": (c_int, [c_vp, c_int, c_int, C.POINTER(c_vp)]),
     "ssq_feeder_destroy": (None, [c_vp]),
     "ssq_feeder_push": (c_int, [c_vp, c_vp, c_i64, C.c_float, c_vp, C.POINTER(c_i64)]),

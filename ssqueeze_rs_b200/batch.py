@@ -329,7 +329,7 @@ class SsqStftStream:
         if transform not in ("ssq_stft", "stft"):
             raise ValueError("transform must be 'ssq_stft' or 'stft'")
         self.eng = engine
-        self.channels, self.n_freqs = int(channels), int(n_fft) // 2 + 1
+        self.channels, self.n_freqs, self.max_chunk = int(channels), int(n_fft) // 2 + 1, int(max_chunk)
         w, wp = _wptr(window)
         h = C.c_void_p()
         st = load().ssq_stream_create_ex(engine.ctx.handle, int(channels), int(n_total), int(max_chunk), wp, len(w),
@@ -361,6 +361,90 @@ class SsqStftStream:
 
     def close(self):
         if self._h:
+            load().ssq_stream_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class CwtStream:
+    """Streaming cwt / ssq_cwt over chunks of an interleaved [samples, channels] recording (int16 or float32 CUDA
+    tensors): the dask `map_overlap(depth=overlap, boundary="reflect")` caller of the reference's CWT scripts
+    (tests/cwt_test.py:117-119,187-193 of the reference), DESIGN §3.6b.  Block b covers output columns
+    [b block, (b + 1) block) and is the reference's call on its extended input x~[b block - overlap, (b + 1) block +
+    overlap) (x~: the recording mirrored with the edge sample repeated at both ends), trimmed to its own columns.
+    `push(chunk)` returns the columns of the blocks that became complete, complex64 [channels, ns, cols]; the result
+    does not depend on how the recording is cut into pushes.  The CWT has no seam-exact stream: a block differs from
+    the whole-signal transform near its seams by an amount that falls with overlap / scale (DESIGN §3.6b).
+
+        cs = CwtStream(eng, 384, n, max_chunk=1 << 18, block=1 << 17, overlap=1 << 14, fs=30000.0)
+        for Tx in RecordingFeeder(eng, rec, None, chunk=1 << 18, scale=0.195, stream=cs):
+            power += Tx.abs().square().sum(dim=2)   # [384, ns]: the reduction stays on the device
+
+    The arguments are those of `Engine.ssq_cwt` (transform="ssq_cwt") and `Engine.cwt` (transform="cwt", l1_norm).
+    scales default to `Engine.default_scales(block + 2 overlap, nv)`, what the reference's call on a full block uses."""
+
+    def __init__(self, engine: "Engine", channels, n_total, max_chunk, block, overlap, wavelet="gmw", scales=None,
+                 fs=None, t=None, nv=32, transform="ssq_cwt", padtype="reflect", squeezing="sum", maprange="peak",
+                 ssq_freqs="log", gamma=None, flipud=True, l1_norm=True):
+        if transform not in ("ssq_cwt", "cwt"):
+            raise ValueError("transform must be 'ssq_cwt' or 'cwt'")
+        self.eng, self.transform = engine, transform
+        self.channels, self.max_chunk = int(channels), int(max_chunk)
+        if scales is None:
+            sc = engine.default_scales(int(block) + 2 * int(overlap), nv) if int(block) >= 1 else np.ones(1)
+        else:
+            sc = scales
+        self.scales = np.ascontiguousarray(sc, dtype=np.float64)
+        self.ns = len(self.scales)
+        dt = float(t[1] - t[0]) if t is not None else (1.0 / float(fs) if fs is not None else 1.0)
+        if transform == "cwt":
+            mode, flags = 2, (0 if l1_norm else _lib.FLAG_L2_NORM)
+        else:
+            mode, flags = 3, (0 if flipud else _lib.FLAG_NO_FLIPUD)
+        h = C.c_void_p()
+        st = load().ssq_stream_create_cwt(engine.ctx.handle, self.channels, int(n_total), self.max_chunk, int(block),
+                                          int(overlap), mode, 1 if wavelet == "morlet" else 0,
+                                          C.c_void_p(self.scales.ctypes.data), self.ns, dt,
+                                          1 if ssq_freqs == "linear" else 0, PAD.get(padtype, 0),
+                                          SQUEEZE.get(squeezing, 0), 1 if maprange == "maximal" else 0,
+                                          float("nan") if gamma is None else float(gamma), flags, C.byref(h))
+        raise_status(st, engine.ctx.handle)
+        self._h = h
+
+    @property
+    def total_frames(self) -> int:
+        """Output columns over the whole recording: n_total."""
+        return int(load().ssq_stream_total_frames(self._h))
+
+    def ssq_freqs(self, last=False):
+        """The ssq grid (float64 [ns]) of the full blocks, or of the last block (its own under maprange="maximal")."""
+        f = np.empty(self.ns, dtype=np.float64)
+        raise_status(load().ssq_stream_ssq_freqs(self._h, 1 if last else 0, C.c_void_p(f.ctypes.data)),
+                     self.eng.ctx.handle)
+        return f
+
+    def push(self, chunk, scale=1.0):
+        import torch
+        assert chunk.is_cuda and chunk.dim() == 2 and chunk.shape[1] == self.channels and chunk.is_contiguous()
+        n_new = chunk.shape[0]
+        cols = max(int(load().ssq_stream_frames_after(self._h, n_new)), 0)
+        out = torch.empty((self.channels, self.ns, cols), dtype=torch.complex64, device=chunk.device)
+        self.eng._bind_stream()
+        fw = C.c_int64()
+        fn = {torch.int16: load().ssq_stream_push_i16, torch.float32: load().ssq_stream_push_f32}[chunk.dtype]
+        st = fn(self._h, C.c_void_p(chunk.data_ptr()), n_new, float(scale),
+                C.c_void_p(out.data_ptr() if cols > 0 else 0), C.byref(fw))
+        raise_status(st, self.eng.ctx.handle)
+        assert fw.value == cols
+        return out
+
+    def close(self):
+        if getattr(self, "_h", None):
             load().ssq_stream_destroy(self._h)
             self._h = None
 
@@ -512,10 +596,15 @@ class RecordingFeeder:
 
         for Sx in RecordingFeeder(eng, rec, win, 512, 32, chunk=1 << 18, scale=0.195, transform="stft"):
             y = inv.push(mask * Sx)      # inv = IstftStream(..., out="i16_interleaved", scale=0.195)
+
+    stream: a `CwtStream` or `SsqStftStream` made for this recording's channels and length; the feeder drives it
+    (chunks of at most its max_chunk) and yields its outputs, [channels, ns or n_freqs, columns]; window and the
+    transform arguments are then unused.  The caller keeps the stream and closes it.
     """
 
     def __init__(self, engine: "Engine", recording, window, n_fft=512, hop_len=32, fs=1.0, chunk=1 << 16, scale=1.0,
-                 padtype="reflect", squeezing="sum", gamma=None, depth=3, transform="ssq_stft", modulated=False):
+                 padtype="reflect", squeezing="sum", gamma=None, depth=3, transform="ssq_stft", modulated=False,
+                 stream=None):
         rec = recording
         if rec.ndim != 2:
             raise ValueError("recording must be [samples, channels]")
@@ -524,9 +613,17 @@ class RecordingFeeder:
         self.eng, self.rec, self.scale = engine, rec, float(scale)
         self.n_total, self.channels = int(rec.shape[0]), int(rec.shape[1])
         self.chunk = int(min(max(1, chunk), self.n_total))
-        self.stream = SsqStftStream(engine, self.channels, self.n_total, self.chunk, window, n_fft, hop_len, fs,
-                                    padtype=padtype, squeezing=squeezing, gamma=gamma, transform=transform,
-                                    modulated=modulated)
+        self._own_stream = stream is None
+        if stream is None:
+            self.stream = SsqStftStream(engine, self.channels, self.n_total, self.chunk, window, n_fft, hop_len, fs,
+                                        padtype=padtype, squeezing=squeezing, gamma=gamma, transform=transform,
+                                        modulated=modulated)
+        else:
+            if stream.channels != self.channels:
+                raise ValueError(f"stream has {stream.channels} channels, the recording {self.channels}")
+            self.stream = stream
+            self.chunk = min(self.chunk, stream.max_chunk)
+        self.rows = self.stream.ns if isinstance(self.stream, CwtStream) else self.stream.n_freqs
         h = C.c_void_p()
         st = load().ssq_feeder_create(self.stream._h, 0 if rec.dtype == np.int16 else 1, int(depth), C.byref(h))
         raise_status(st, engine.ctx.handle)
@@ -548,7 +645,7 @@ class RecordingFeeder:
             src = np.ascontiguousarray(src)
         frames = max(int(load().ssq_stream_frames_after(self.stream._h, n_new)), 0)
         # (torch's caching allocator hands the same blocks back once the consumer drops the previous chunks)
-        out = torch.empty((self.channels, self.stream.n_freqs, frames), dtype=torch.complex64, device=self.eng.device)
+        out = torch.empty((self.channels, self.rows, frames), dtype=torch.complex64, device=self.eng.device)
         self.eng._bind_stream()
         fw = C.c_int64()
         st = load().ssq_feeder_push(self._h, C.c_void_p(src.ctypes.data), n_new, self.scale,
@@ -569,7 +666,7 @@ class RecordingFeeder:
         if getattr(self, "_h", None):
             load().ssq_feeder_destroy(self._h)
             self._h = None
-        if getattr(self, "stream", None):
+        if getattr(self, "stream", None) and getattr(self, "_own_stream", True):
             self.stream.close()
 
     def __enter__(self):

@@ -24,9 +24,10 @@
 struct SsqCwtParams {
   const float2* W;    // [ns, n] (stand-alone kernel only)
   const float2* D;
-  float2* Tx;         // stand-alone: [ns, n] of one channel; fused: [channels, ns, n]; zero-initialised
+  float2* Tx;         // stand-alone: [ns, pitch] of one channel; fused: [channels, ns, pitch]; zero-initialised
   int ns;
-  int64_t n;
+  int64_t n;          // columns written per row (fused: per (channel, block) row; stand-alone: per thread sweep)
+  int64_t pitch;      // row pitch of Tx (n for the batch call; the push's column count for a stream)
   float gate;         // gamma / K (in the units of the W handed to ssq_cwt_item): |W| < gate -> skipped
   float gate2f;       // max(gate^2, 1e-30), at most 3e38: below it (or above 1e30) the exact out-of-line path decides
   int is_log;
@@ -114,7 +115,7 @@ __global__ void ssq_cwt_reassign_kernel(const SsqCwtParams P) {
       if (P.aux_kb) P.aux_kb[(size_t)(i0 + u) * P.n + b] = k;
       if (P.aux_w) P.aux_w[(size_t)(i0 + u) * P.n + b] = w;
       if (k < 0) continue;
-      float2* t = Tc + (size_t)k * P.n;
+      float2* t = Tc + (size_t)k * P.pitch;
       if (P.squeezing == SSQ_SQUEEZE_LEBESGUE) atomicAdd(&t->x, P.leb_val);
       else atomicAdd(t, make_float2(Wb[u].x * P.K, Wb[u].y * P.K));
     }
@@ -156,16 +157,32 @@ struct FftPass {
   // mode 6: rows of fr_nfft points with row stride fr_ld inside rows of L: in[row * fr_ld + idx] (conjugated when
   // conj_in) * fr_chirp[idx] (when given), zero beyond fr_nfft (icwt two-integral branch at any row length)
   int conj_in;
+  // ---- CWT stream (cwt_host.inl, CwtBlocks) -----------------------------------------
+  // x-hat row r of a stream call is block blk_first + r % blk_nb of channel r / blk_nb; blk_nb == 0 is the batch call
+  // (row r is channel r).  Load mode 1 reads the block's extended input e[j] = x~[b C - d + j] (x~: the recording
+  // mirrored with the edge sample repeated) from x (rows of x_stride, recording position rec_origin at column 0);
+  // store modes 1 and 2 write row (channel, scale) of an output of out_pitch columns from column out_col0 + bl C.
+  int blk_nb;
+  int64_t blk_C, blk_d, blk_first, rec_n, rec_origin;
+  int64_t out_pitch, out_col0;
   // ---- store functor ------------------------------------------------------------
   int store_mode;     // 0 plain, 1 final: scaled, unpadded rows to outW / outD, 2: fused ssq_cwt epilogue
   float2* outW;       // [channels, ns, out_cols]
   float2* outD;       // [channels, ns, out_cols] (may be NULL)
-  int64_t out_cols, n1;  // out_cols = n (unpadded) or L (rpadded, n1 = 0)
+  int64_t out_cols, n1;  // columns [n1, n1 + out_cols) of the padded row: n (unpadded) or L (rpadded, n1 = 0)
   float out_scale;    // K / L   (K = de-normalisation constant of psi-hat)
   int l2_norm;
   // ---- fused ssq_cwt epilogue (store_mode 2, fft128_pass_kernel<TC, true> only) ------------------
-  SsqCwtParams E;     // E.Tx: [channels, ns, n]
+  SsqCwtParams E;     // E.Tx: [channels, ns, E.pitch]
 };
+
+// Element offset of column 0 of row cs = (x-hat row) * ns + scale in an output of `pitch` columns per row
+__device__ __forceinline__ size_t cwt_out_offset(const FftPass& P, unsigned cs, int64_t pitch) {
+  if (P.blk_nb == 0) return (size_t)cs * pitch;
+  const unsigned rb = cs / (unsigned)P.ns, si = cs - rb * (unsigned)P.ns;
+  const unsigned ch = rb / (unsigned)P.blk_nb, bl = rb - ch * (unsigned)P.blk_nb;
+  return ((size_t)ch * P.ns + si) * pitch + P.out_col0 + (size_t)bl * P.blk_C;
+}
 
 // GMW(gamma=3, beta=60) is evaluated as exp(60 ln w - w^3 - SSQ_GMW_LOGPEAK): peak 1
 // instead of the reference's un-normalised 2*exp(...) (~4e17, cwt.rs:536-541), which
@@ -200,9 +217,27 @@ __device__ __forceinline__ float psihat(int wavelet, float w) {
   return expf(60.f * logf(w) - w * w * w - (float)SSQ_GMW_LOGPEAK);
 }
 
-__device__ __forceinline__ float cwt_sample(const FftPass& P, int ch, int64_t p, int64_t L) {
+// Stream call: the reference's pad of the extended block input e (length P.n), then e[j] = x~[b C - d + j] with the
+// symmetric fold at the recording ends (x~[q] = x[-1 - q], q < 0; x[2 N - 1 - q], q >= N: np.pad mode "symmetric",
+// dask's boundary="reflect"), read in place from the carry-over buffer.  d <= C and d <= N: one fold suffices.
+__device__ __forceinline__ float cwt_block_sample(const FftPass& P, int64_t g, int64_t p, int64_t L) {
+  int64_t o = p - (L - P.n) / 2;
+  if (o < 0 || o >= P.n) {
+    if (P.padtype == SSQ_PAD_ZERO) return 0.f;
+    o = o < 0 ? -o : 2 * P.n - 2 - o;
+    if (o < 0 || o >= P.n) return 0.f;
+  }
+  const int64_t ch = g / P.blk_nb, b = P.blk_first + (g - ch * P.blk_nb);
+  int64_t q = b * P.blk_C - P.blk_d + o;
+  if (q < 0) q = -1 - q;
+  else if (q >= P.rec_n) q = 2 * P.rec_n - 1 - q;
+  return __ldg(P.x + (size_t)ch * P.x_stride + (q - P.rec_origin));
+}
+
+__device__ __forceinline__ float cwt_sample(const FftPass& P, int64_t g, int64_t p, int64_t L) {
+  if (P.blk_nb) return cwt_block_sample(P, g, p, L);
   // utils/array.rs:52-98: left = (L-n)/2
-  const float* x = P.x + (size_t)ch * P.x_stride;
+  const float* x = P.x + (size_t)g * P.x_stride;
   const int64_t left = (L - P.n) / 2;
   const int64_t o = p - left;
   if (o >= 0 && o < P.n) return __ldg(x + o);
@@ -219,7 +254,7 @@ __device__ __forceinline__ float2 pass_load(const FftPass& P, int row, int64_t i
   const int64_t L = (int64_t)1 << P.log2L;
   if (P.load_mode == 0) return P.in[(size_t)row * L + idx];
   const int64_t g = P.row0 + row;
-  if (P.load_mode == 1) return make_float2(cwt_sample(P, (int)g, idx, L), 0.f);
+  if (P.load_mode == 1) return make_float2(cwt_sample(P, g, idx, L), 0.f);
   if (P.load_mode == 4) return cmulf(P.in[(size_t)row * L + idx], __ldg(P.mul + idx));
   if (P.load_mode == 6) {
     if (idx >= P.fr_nfft) return make_float2(0.f, 0.f);
@@ -282,7 +317,7 @@ __device__ __forceinline__ void pass_store(const FftPass& P, int row, int64_t o,
   float s = P.out_scale;
   if (P.l2_norm) s *= sqrtf(__ldg(P.scales + (int)(cs % P.ns)));  // cwt.rs:253
   float2* dst = which ? P.outD : P.outW;
-  dst[(size_t)cs * P.out_cols + col] = make_float2(v.x * s, v.y * s);
+  dst[cwt_out_offset(P, (unsigned)cs, P.out_pitch) + col] = make_float2(v.x * s, v.y * s);
 }
 
 // grid: (L / (R*T), rows).  Dynamic smem: 2 * R * T float2.
@@ -423,7 +458,8 @@ __global__ void __launch_bounds__(8 * TC) fft128_pass_kernel(const FftPass P) {
   if (FUSED && threadIdx.x == 128) {
     const unsigned cs0 = ((unsigned)P.row0 + 2u * blockIdx.y) >> 1;  // channel * ns + scale (rows: channel, scale, which)
     const unsigned chn0 = cs0 / (unsigned)P.E.ns;
-    s_tch = P.E.Tx + (size_t)chn0 * P.E.ns * P.E.n + (P.E.flipud ? (size_t)(P.E.ns - 1) * P.E.n : (size_t)0);
+    s_tch = P.E.Tx + cwt_out_offset(P, chn0 * (unsigned)P.E.ns, P.E.pitch) +
+            (P.E.flipud ? (size_t)(P.E.ns - 1) * P.E.pitch : (size_t)0);
     s_drow = (size_t)cs0 * P.E.n;
   }
   // in-row indices are 32-bit (L <= 2^27, checked on the host): the passes are issue-bound and 64-bit
@@ -579,8 +615,8 @@ __global__ void __launch_bounds__(8 * TC) fft128_pass_kernel(const FftPass P) {
     const int base = ((j - kk) << 7) + kk - (int)P.n1;
     const int koff = g + 8 * which_l;
     // row of Tx = flipud ? ns - 1 - bin : bin, as a signed 32-bit element offset from a per-channel base (the host
-    // takes this path only while ns * n < 2^31): one integer multiply-add per item
-    const int rstep = P.E.flipud ? -(int)P.E.n : (int)P.E.n;
+    // takes this path only while ns * pitch < 2^31): one integer multiply-add per item
+    const int rstep = P.E.flipud ? -(int)P.E.pitch : (int)P.E.pitch;
     float2* Tch = s_tch;
     const size_t drow = s_drow;  // diagnostics: [channels, ns, n]
     const bool diag = P.E.aux_kb != nullptr || P.E.aux_w != nullptr;
@@ -620,7 +656,7 @@ __global__ void __launch_bounds__(8 * TC) fft128_pass_kernel(const FftPass P) {
   if (P.store_mode == 1) {
     const unsigned gr = (unsigned)P.row0 + (unsigned)row;
     const unsigned cs = gr / (unsigned)P.nd;  // channel * ns + scale
-    sdst = ((gr - cs * (unsigned)P.nd) ? P.outD : P.outW) + (size_t)cs * P.out_cols;
+    sdst = ((gr - cs * (unsigned)P.nd) ? P.outD : P.outW) + cwt_out_offset(P, cs, P.out_pitch);
     sscale = P.out_scale;
     if (P.l2_norm) sscale *= sqrtf(__ldg(P.scales + (int)(cs % (unsigned)P.ns)));  // cwt.rs:253
     soff = (int)P.n1;

@@ -1011,9 +1011,15 @@ struct ssq_stream {
   int64_t channels, n_total, max_chunk, cap;
   std::vector<double> wfit;
   int n_fft, hop, left, padtype, squeezing;
-  int mode = 0;        // 0 ssq_stft, 1 stft
-  unsigned flags = 0;  // SSQ_FLAG_MODULATED (ssq_stft)
+  int mode = 0;        // 0 ssq_stft, 1 stft, 2 cwt, 3 ssq_cwt (ssq_stream_create_cwt, cwt_host.inl)
+  unsigned flags = 0;  // SSQ_FLAG_MODULATED (ssq_stft), SSQ_FLAG_L2_NORM (cwt), SSQ_FLAG_NO_FLIPUD (ssq_cwt)
   double fs, gamma;
+  // CWT modes: frames are output columns, computed in blocks of `block` columns with `overlap` samples of context on
+  // either side (DESIGN §3.6b)
+  int64_t block = 0, overlap = 0, pitch_bound = 0;
+  int wavelet = 0, freq_dist = 0, maprange = 0;
+  std::vector<double> scales;
+  double dt = 1.0;
   int64_t n_frames_total;
   int64_t received = 0;   // samples pushed so far
   int64_t origin = 0;     // global index of buf[.][0]
@@ -1041,11 +1047,42 @@ __global__ void deinterleave_kernel(const T* __restrict__ in, int64_t n_new, int
 
 static int64_t stream_frames_ready(const ssq_stream* s, int64_t received) {
   if (received >= s->n_total) return s->n_frames_total;
+  if (s->mode >= 2) {  // block b is ready once min(N, (b + 1) C + d) samples have arrived
+    const int64_t r = received - s->overlap;
+    return r < s->block ? 0 : r / s->block * s->block;
+  }
   const int64_t a = received - s->n_fft + s->left;  // last frame f with f*hop - left + n_fft - 1 < received
   // frame 0 also reads x[left] through the left reflection: in upstream framing with even n_fft that is one sample
   // past its own last one (left = n_fft - left), so with received == left it is not ready yet
   if (a < 0 || received <= s->left) return 0;
   return std::min<int64_t>(s->n_frames_total, a / s->hop + 1);
+}
+
+// The two [channels, cap] carry-over buffers of a new stream; on failure the stream is destroyed.
+static ssq_status stream_buffers(ssq_stream* s) {
+  ssq_ctx* ctx = s->ctx;
+  for (int i = 0; i < 2; ++i) {
+    cudaError_t e = cudaMalloc((void**)&s->buf[i], (size_t)s->channels * s->cap * sizeof(float));
+    if (e != cudaSuccess) {
+      (void)cudaGetLastError();
+      if (s->buf[0]) cudaFree(s->buf[0]);
+      const long long ch = (long long)s->channels, cap = (long long)s->cap;
+      delete s;
+      return ssq_fail(ctx, SSQ_ENOMEM, "stream buffers (%lld x %lld floats): %s", ch, cap, cudaGetErrorString(e));
+    }
+  }
+  // stft mode pairs frames in one complex FFT: the partner of the last ready frame reads samples not received yet.
+  // Its values only reach the real frame through the rounding of the split, unless they are huge or NaN, which
+  // never-written device memory (freed by an earlier user in this process) can hold.
+  for (int i = 0; i < 2; ++i) {
+    cudaError_t e = cudaMemsetAsync(s->buf[i], 0, (size_t)s->channels * s->cap * sizeof(float), ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) {
+      ssq_stream_destroy(s);
+      return ssq_fail(ctx, SSQ_ECUDA, "stream buffers: %s", cudaGetErrorString(e));
+    }
+  }
+  return SSQ_OK;
 }
 
 extern "C" ssq_status ssq_stream_create(ssq_ctx* ctx, int64_t channels, int64_t n_total, int64_t max_chunk,
@@ -1096,27 +1133,7 @@ extern "C" ssq_status ssq_stream_create_ex(ssq_ctx* ctx, int64_t channels, int64
   s->gamma = gamma;
   s->n_frames_total = (n_total - 1) / hop + 1;
   s->cap = max_chunk + n_fft + hop + 32;
-  for (int i = 0; i < 2; ++i) {
-    cudaError_t e = cudaMalloc((void**)&s->buf[i], (size_t)channels * s->cap * sizeof(float));
-    if (e != cudaSuccess) {
-      (void)cudaGetLastError();
-      if (s->buf[0]) cudaFree(s->buf[0]);
-      delete s;
-      return ssq_fail(ctx, SSQ_ENOMEM, "stream buffers (%lld x %lld floats): %s", (long long)channels,
-                      (long long)s->cap, cudaGetErrorString(e));
-    }
-  }
-  // stft mode pairs frames in one complex FFT: the partner of the last ready frame reads samples not received yet.
-  // Its values only reach the real frame through the rounding of the split, unless they are huge or NaN, which
-  // never-written device memory (freed by an earlier user in this process) can hold.
-  for (int i = 0; i < 2; ++i) {
-    cudaError_t e = cudaMemsetAsync(s->buf[i], 0, (size_t)channels * s->cap * sizeof(float), ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-      ssq_stream_destroy(s);
-      return ssq_fail(ctx, SSQ_ECUDA, "stream buffers: %s", cudaGetErrorString(e));
-    }
-  }
+  SSQ_TRY(stream_buffers(s));
   *out = s;
   return SSQ_OK;
 }
@@ -1137,6 +1154,8 @@ extern "C" int64_t ssq_stream_frames_after(const ssq_stream* s, int64_t n_new) {
   const int64_t r = std::min<int64_t>(s->n_total, s->received + n_new);
   return stream_frames_ready(s, r) - s->f_next;
 }
+
+static ssq_status cwt_stream_run(ssq_stream* s, const float* buf, int64_t c0, int64_t c1, float2* out);  // cwt_host.inl
 
 template <typename T>
 static ssq_status stream_push(ssq_stream* s, const T* d_chunk, int64_t n_new, float scale, float* d_Tx,
@@ -1166,28 +1185,32 @@ static ssq_status stream_push(ssq_stream* s, const T* d_chunk, int64_t n_new, fl
   const int64_t count = f_end - s->f_next;
   if (count > 0) {
     if (!d_Tx) return ssq_fail(ctx, SSQ_EINVAL, "d_Tx is NULL but %lld frames are ready", (long long)count);
-    StftCall c;
-    c.mode = s->mode;
-    c.d_x = buf;
-    c.x_origin = s->origin;
-    c.channels = s->channels;
-    c.n = s->n_total;
-    c.x_stride = s->cap;
-    c.wfit = s->wfit;
-    c.n_fft = s->n_fft;
-    c.hop = s->hop;
-    c.fs = s->mode == 1 ? 1.0 : s->fs;
-    c.padtype = s->padtype;
-    c.squeezing = s->mode == 1 ? SSQ_SQUEEZE_SUM : s->squeezing;
-    c.gamma = s->mode == 1 ? 0.0 : s->gamma;
-    c.flags = s->flags;
-    c.d_out = (float2*)d_Tx;
-    c.aux_Sx = nullptr;
-    c.aux_dSx = nullptr;
-    c.aux_w = nullptr;
-    c.frame0 = s->f_next;
-    c.n_frames_call = count;
-    SSQ_TRY(run_stft_family(ctx, c));
+    if (s->mode >= 2) {
+      SSQ_TRY(cwt_stream_run(s, buf, s->f_next, f_end, (float2*)d_Tx));
+    } else {
+      StftCall c;
+      c.mode = s->mode;
+      c.d_x = buf;
+      c.x_origin = s->origin;
+      c.channels = s->channels;
+      c.n = s->n_total;
+      c.x_stride = s->cap;
+      c.wfit = s->wfit;
+      c.n_fft = s->n_fft;
+      c.hop = s->hop;
+      c.fs = s->mode == 1 ? 1.0 : s->fs;
+      c.padtype = s->padtype;
+      c.squeezing = s->mode == 1 ? SSQ_SQUEEZE_SUM : s->squeezing;
+      c.gamma = s->mode == 1 ? 0.0 : s->gamma;
+      c.flags = s->flags;
+      c.d_out = (float2*)d_Tx;
+      c.aux_Sx = nullptr;
+      c.aux_dSx = nullptr;
+      c.aux_w = nullptr;
+      c.frame0 = s->f_next;
+      c.n_frames_call = count;
+      SSQ_TRY(run_stft_family(ctx, c));
+    }
     s->f_next = f_end;
   }
   if (frames_written) *frames_written = std::max<int64_t>(count, 0);
@@ -1195,8 +1218,10 @@ static ssq_status stream_push(ssq_stream* s, const T* d_chunk, int64_t n_new, fl
   if (s->f_next < s->n_frames_total) {
     // the next frame starts at f_next*hop - left; frames that touch the right padding also read the
     // reflected samples x[2n-2-o] >= n - n_fft, which may lie before their own start when hop is large
-    const int64_t want = std::min<int64_t>(std::max<int64_t>(0, s->f_next * s->hop - s->left),
-                                           std::max<int64_t>(0, s->n_total - s->n_fft));
+    // (CWT: the next block reads x~[f_next - d, ...); its reflections at the recording ends lie inside that range)
+    const int64_t want = s->mode >= 2 ? std::max<int64_t>(0, s->f_next - s->overlap)
+                                      : std::min<int64_t>(std::max<int64_t>(0, s->f_next * s->hop - s->left),
+                                                          std::max<int64_t>(0, s->n_total - s->n_fft));
     const int64_t new_origin = std::max<int64_t>(s->origin, want);
     if (new_origin > s->origin) {
       const int64_t keep = s->received - new_origin;
