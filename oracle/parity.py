@@ -208,8 +208,8 @@ def emulate_fp32_kernel(x, window, n_fft, hop, fs, padtype="reflect", gamma=None
 C_CWT = 128.0
 
 
-def cwt_bin_tolerance(aux_o, x, wavelet, dt, padtype, ssq_freqs):
-    Wx, dWx, w_o, scales = aux_o["Wx"], aux_o["dWx"], aux_o["w"], aux_o["scales"]
+def cwt_row_errors(Wx, dWx, x, wavelet, scales, dt, padtype):
+    """(e_W, e_D) per row of Wx, dWx: the fp32 error bound of each row (see above)."""
     ns, N = Wx.shape
     L = O.next_power_of_2(N + N // 2)
     padded = O.pad_zero_cwt(x, L) if padtype == "zero" else O.pad_reflect_cwt(np.asarray(x, dtype=np.float64), L)
@@ -226,8 +226,14 @@ def cwt_bin_tolerance(aux_o, x, wavelet, dt, padtype, ssq_freqs):
     # its peak (cwt_kernels.cuh psihat); the dropped tail is at most floor * sum_k |x-hat_k| / L in W
     xh1 = float(np.abs(np.fft.fft(padded)).sum()) / L
     floor_rel, peak = (2.2e-16, 1.0622519320271968) if wavelet == "morlet" else (2.0e-18, 2.0 * math.exp(39.914641217580179))
-    eW = eW + floor_rel * peak * xh1
-    eD = eD + floor_rel * peak * xh1 * (math.pi / dt)
+    return eW + floor_rel * peak * xh1, eD + floor_rel * peak * xh1 * (math.pi / dt)
+
+
+def cwt_bin_tolerance(aux_o, x, wavelet, dt, padtype, ssq_freqs, row_err=None):
+    """row_err: (e_W, e_D) of the rows, when aux_o holds a slice of columns of them (`cwt_row_errors` needs whole
+    rows)."""
+    Wx, dWx, w_o, scales = aux_o["Wx"], aux_o["dWx"], aux_o["w"], aux_o["scales"]
+    eW, eD = row_err if row_err is not None else cwt_row_errors(Wx, dWx, x, wavelet, scales, dt, padtype)
     aW = np.abs(Wx)
     with np.errstate(over="ignore", invalid="ignore", divide="ignore"):
         # delta(dW / W) <= (e_D + |dW / W| e_W) / (|W| - e_W): unbounded once |W| is within the error itself
@@ -240,16 +246,18 @@ def cwt_bin_tolerance(aux_o, x, wavelet, dt, padtype, ssq_freqs):
     return np.nan_to_num(dw_abs, nan=np.inf, posinf=np.inf), is_log, eW
 
 
-def classify_cwt_bins(kb_dev, aux_o, x, wavelet, dt, padtype, ssq_freqs, flipud=True, gamma=None, w_dev=None):
+def classify_cwt_bins(kb_dev, aux_o, x, wavelet, dt, padtype, ssq_freqs, flipud=True, gamma=None, w_dev=None,
+                      row_err=None):
     """kb_dev: int [ns, N]: destination ROW of Tx for every (scale, column), -1 where nothing was added (gated,
-    non-finite w, out of range).  aux_o: oracle aux (Wx, dWx, w, k, scales)."""
+    non-finite w, out of range).  aux_o: oracle aux (Wx, dWx, w, k, scales), or a slice of its columns with
+    row_err = (e_W, e_D) of the whole rows (`cwt_row_errors`)."""
     Wx, w_o, k_o = aux_o["Wx"], aux_o["w"], aux_o["k"]
     ns, N = Wx.shape
     nf = len(ssq_freqs)
     kb_dev = np.asarray(kb_dev).astype(np.int64)
     assert kb_dev.shape == k_o.shape
     g = 10.0 * O.EPS64 if gamma is None else float(gamma)
-    dw_abs, is_log, eW = cwt_bin_tolerance(aux_o, x, wavelet, dt, padtype, ssq_freqs)
+    dw_abs, is_log, eW = cwt_bin_tolerance(aux_o, x, wavelet, dt, padtype, ssq_freqs, row_err)
     if is_log:
         f0 = math.log2(ssq_freqs[0])
         step = (math.log2(ssq_freqs[nf - 1]) - f0) / (nf - 1.0) if nf > 1 else 1.0

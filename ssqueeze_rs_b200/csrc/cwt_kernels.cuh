@@ -522,8 +522,13 @@ __global__ void __launch_bounds__(8 * TC) fft128_pass_kernel(const FftPass P) {
     const float2* xh = P.xhat + (size_t)chn * L;
     const float cut = P.wavelet == SSQ_WAVELET_MORLET ? 14.5f : 4.5f;
     const float inv_L = 1.f / (float)L;
+    // (the bound is compared in float but kept as an int: (float)(L / 2 + 1) rounds down to L / 2 from L = 2^25 on,
+    // which dropped the Nyquist bin of rows whose band reaches it)
     int blim = (L >> 1) + 1;  // negative frequencies: psi-hat = 0 (cwt.rs:496-541)
-    if (scale > 0.f) blim = (int)fminf((float)blim, cut * (float)L / (6.283185307179586f * scale) * 1.0001f + 2.f);
+    if (scale > 0.f) {
+      const float b = cut * (float)L / (6.283185307179586f * scale) * 1.0001f + 2.f;
+      if (b < (float)blim) blim = (int)b;
+    }
 #pragma unroll
     for (int u = 0; u < 16; ++u) {
       const int idx = (j + (g + 8 * u) * Q) >> P.up_shift;
